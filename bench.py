@@ -2,6 +2,7 @@
 """bench.py — QR GFLOP/s (fp64) of qr! on the BASELINE workload, one JSON line on rank 0.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 3|2] [--m M --n N --nb NB]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -20,6 +21,9 @@ the N GPUs (strong scaling: total work fixed).  A "step" is one full factorisati
              whole sweep) and LAPACK dgeqrf, the reference tests' own normaliser (test/runtests.jl:49,53-54).
 --config 2 measures BASELINE configs[1] (8192 x 1024, nb = 1: the unblocked column loop) with an HBM roofline instead.
 --impl reference times the CPU restatement alone (the reference is Julia; Julia is not installed) on the same config.
+--dump-outputs DIR writes what the last timed qr! handed back, as float64 .npy files, so that two builds can be compared
+output for output (the inputs depend on the arguments only): DIR/alpha.npy (n) and DIR/A.npy (m x k), the factored A at
+the columns of `dump_columns` (all n when the factor fits in 48 MiB, else a fixed seeded sample of k columns).
 """
 import argparse
 import json
@@ -291,6 +295,8 @@ def run_ours(args):
     value = flops / (ms_per_step * 1e-3) / 1e9
     launches_all = int(sumover(float(launches)))
     last = pool[(K - 1) % pool_n]                 # the last timed factorisation (alpha belongs to it)
+    # taken before the legs below refactor pool[0] into the same alpha
+    outputs = gather_outputs(torch, dist, last, alpha, m, n, c0, nl, world, dev) if args.dump_outputs else None
 
     # ---- parity of the last timed factorisation ------------------------------------------------------------------------
     parity = {"tolerance": 1e-13, "oracle_pin": ORACLE_PIN}
@@ -473,6 +479,11 @@ def run_ours(args):
                                 "wide_redone": h.get_option("wide_redone"), "baseline_config": args.config},
                "clocks": clocks, "gpu_launches": launches_all, "e2e": e2e, "roofline": roof, "cpu_baseline": cpu,
                "solve": solve, "parity": parity}
+        if outputs is not None:
+            import numpy as np
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in outputs.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
         print(json.dumps(out))
     if world > 1:
         D.shutdown_distributed()
@@ -515,6 +526,33 @@ def dist_residual(torch, dist, D, Hloc, alpha, m, n, c0, nl, world, rank, dev, h
         dist.all_reduce(t)
         num, den = float(t[0].item()), float(t[1].item())
     return (num / den) ** 0.5
+
+
+DUMP_A_BYTES = 48 << 20          # keeps a dump under 64 MB with alpha (8n bytes) beside it
+
+
+def dump_columns(m, n):
+    """Global columns of the factored A that --dump-outputs writes: all of them when they fit in DUMP_A_BYTES, else a
+    sorted sample drawn with a fixed seed, so that every run with the same m and n writes the same columns."""
+    import numpy as np
+    k = min(n, max(1, DUMP_A_BYTES // (8 * m)))
+    if k == n:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+
+
+def gather_outputs(torch, dist, Hloc, alpha, m, n, c0, nl, world, dev):
+    """The arrays qr!(A) hands back, as host arrays: the factored A at the columns of dump_columns, and alpha (replicated
+    on every rank).  Each rank fills the sampled columns it owns and a sum over ranks assembles them."""
+    cols = dump_columns(m, n)
+    S = torch.zeros(m, len(cols), dtype=torch.float64, device=dev)
+    mine = [(s, int(j) - c0) for s, j in enumerate(cols) if c0 <= j < c0 + nl]
+    if mine:
+        dst, src = zip(*mine)
+        S[:, list(dst)] = Hloc[:, list(src)]
+    if world > 1:
+        dist.all_reduce(S)
+    return {"A": S.cpu().numpy(), "alpha": alpha.cpu().numpy()}
 
 
 def dgemm_peak(torch, dev, nn=8192):
@@ -575,7 +613,13 @@ def main():
     ap.add_argument("--no-solve", action="store_true")
     ap.add_argument("--split", default="even", choices=["even", "balanced"],
                     help="column blocks: DArray default (even) or the reference's load-balanced contiguous split (T:35), rounded to panels")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the factored A (column sample) and alpha of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours: the reference arm times a strided sample of the column sweep, not a whole qr!")
     dm, dn, dnb = (8192, 1024, 1) if args.config == 2 else (32768, 4096, 0)
     args.m, args.n = args.m or dm, args.n or dn
     args.nb = dnb if args.nb < 0 else args.nb

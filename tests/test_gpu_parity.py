@@ -426,3 +426,20 @@ def test_full_size_properties(D, dev, coracle, mn):
     A3.copy_(A2)
     H3 = D.qr_(A3, nb=1)
     assert float((H3.α - H.α[:256]).abs().max() / H.α.abs().max()) < TOL_A
+
+
+# ---- bench.py --dump-outputs: what the timed qr! handed back -----------------------------------------
+def test_bench_dump_outputs_are_the_factorisation(tmp_path, coracle):
+    import json, subprocess, sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    m, n = 2048, 256
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--gpus", "1", "--steps", "3", "--warmup", "3", "--m", str(m),
+                          "--n", str(n), "--no-e2e", "--no-cpu", "--no-solve", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-2000:]
+    assert json.loads(out.stdout.strip().splitlines()[-1])["steps"] == 3
+    A, alpha = np.load(tmp_path / "A.npy"), np.load(tmp_path / "alpha.npy")
+    assert A.shape == (m, n) and A.dtype == np.float64 and alpha.shape == (n,)    # small enough to be written whole
+    Href, aref = coracle.qr(coracle.fill_uniform(0, m, n))
+    assert np.abs(A - Href).max() < TOL_H
+    assert np.abs(alpha - aref).max() < TOL_A * np.abs(aref).max()

@@ -122,3 +122,25 @@ def test_balanced_splits_follow_the_reference_formulas():
 
     imb = lambda w: w.max() / w.mean()
     assert imb(work(D.balanced_splits(P, n))) < 1.1 < imb(work(D.splits(P, n))) < imb(work(D.balanced_splits(P, n, "upstream")))
+
+
+def test_bench_dump_columns_are_fixed_and_within_budget():
+    """--dump-outputs writes the same seeded column sample of the factored A on every run with the same shape, at most
+    48 MiB of it, and assembles it from DArray-style column blocks exactly as from the whole matrix."""
+    import os, sys
+    sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+    import bench
+    assert np.array_equal(bench.dump_columns(2048, 256), np.arange(256))
+    cols = bench.dump_columns(32768, 4096)
+    assert np.array_equal(cols, bench.dump_columns(32768, 4096)) and 32768 * len(cols) * 8 <= bench.DUMP_A_BYTES
+    assert len(set(cols.tolist())) == len(cols) and np.all(np.diff(cols) > 0) and cols[-1] < 4096
+    m, n = 9000, 1000
+    H = D.colmajor_empty(m, n, device="cpu")
+    H.copy_(torch.rand(m, n, dtype=torch.float64))
+    alpha = torch.rand(n, dtype=torch.float64)
+    whole = bench.gather_outputs(torch, None, H, alpha, m, n, 0, n, 1, "cpu")
+    sel = bench.dump_columns(m, n)
+    assert len(sel) < n and np.array_equal(whole["A"], H.numpy()[:, sel]) and np.array_equal(whole["alpha"], alpha.numpy())
+    b = D.splits(3, n)
+    parts = [bench.gather_outputs(torch, None, H[:, b[r]:b[r + 1]], alpha, m, n, b[r], b[r + 1] - b[r], 1, "cpu")["A"] for r in range(3)]
+    assert np.array_equal(sum(parts), whole["A"])
