@@ -100,72 +100,51 @@ static int load_nccl() {
 // ------------------------------------------------------------------------------------------------
 static inline int64_t rup(int64_t x, int64_t a) { return (x + a - 1) / a * a; }
 
+static constexpr int CU_STREAMS = 3;   // catch-up streams of dhqr_qr_host_f64, each with its own V buffer and workspace set
+
 struct dhqr_context {
     int device = 0, sms = 0;
     int rank = 0, nranks = 1;
     ncclComm_t comm = nullptr;
     // options
-    int nb = 128, panel_ctas = 0, sync = 0, panel_backoff = 0, vta_max_chunks = 0, panel_levels = 2;
+    int nb = 128, sync = 0;
     // workspace
     // three V buffers (panels k, k+1 and the one being broadcast live at the same time under look-ahead) and two
     // workspace sets (set 0: trailing update on the caller's stream; set 1: panel chain on the high-priority stream)
-    double* vpk2[6] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr}; size_t vpk_elems[6] = {0, 0, 0, 0, 0, 0}; int64_t vrows_cap = 0;   // packed V [chunk][128][68]; [3..5]: catch-up of late column chunks (host entry)
+    double* vpk2[3 + CU_STREAMS] = {}; size_t vpk_elems[3 + CU_STREAMS] = {}; int64_t vrows_cap = 0;   // packed V [chunk][128][68]; [3..]: catch-up of late column chunks (host entry)
     struct WSet {
         double* wpart = nullptr; size_t wpart_elems = 0;                // gemm_vta partials
         double* wsum = nullptr;  size_t wsum_elems = 0;                 // reduced Wext
         double* ypk = nullptr;   size_t ypk_elems = 0;                  // packed Y = -T'W
         double* linv = nullptr;  size_t linv_elems = 0;                 // [128*128]
-    } ws[6];                                                            // [2]: the chain's second apply (columns of panel k+2) on its own stream; [3..5]: catch-up (host entry)
+    } ws[3 + CU_STREAMS];                                               // [2]: the chain's second apply (columns of panel k+2) on its own stream; [3..]: catch-up (host entry)
     double* linv_all = nullptr; size_t linv_all_elems = 0;              // T' of every outer panel of the factorisation in flight (look-ahead): slot k = panel k
     double* tslot(int k) const { return linv_all + (size_t)k * 128 * 128; }
-    cudaStream_t hp_stream = nullptr;                                   // stream of the panel chain (high priority by default)
-    cudaStream_t hp_hi = nullptr, hp_lo = nullptr;
+    cudaStream_t hp_stream = nullptr;                                   // stream of the panel chain (high priority)
     cudaStream_t comm_stream = nullptr;                                 // collectives of the look-ahead schedule (high priority)
     cudaStream_t aux_stream = nullptr;                                  // small side kernels of the wide chain (Rt = R2 R1, k_trecon), high priority
     cudaEvent_t ev_aux[4] = {nullptr, nullptr, nullptr, nullptr};
-    int wide_aux = 1;                                                   // option: run them beside the chain instead of inside it
     cudaStream_t hp2_stream = nullptr;                                  // the chain's second apply (V_k -> columns of panel k+2), high priority
-    int wide_trecon = 1;                                                // option: T' of a wide panel from the reconstruction (k_trecon)
     int host_trace = 0;                                                 // option: print a stage timeline of dhqr_qr_host_f64 to stderr
-    int hp2 = 1;                                                        // option: use it (0: that apply stays on the chain's stream)
     int lookahead = 1;
-    int la_trace = 0;                                                   // keep timing events of the look-ahead schedule
-    std::vector<float> la_times;                                        // [k][3]: panel k done (hp), next k signalled (st), bulk k done (st), ms since start
     unsigned long long* cells = nullptr;                                // panel exchange cells [IB+1][MAXG+1][IB][2]
     uint32_t ll_epoch = 0;
     unsigned long long* cells2 = nullptr;                               // exchange cells of the panel kernel's fast path
     int* fast_stats = nullptr;                                          // [2] fast / fallback panel counters
     int panel_fast = 1;
-    unsigned int* sm_ticket = nullptr;                                  // per-SM counters for gemm_cvy phase staggering
-    int cvy_stagger = 0;
-    int bs_wave = 1;                                                    // back-substitution as one wavefront launch per right-hand side
     int bs_wave_max_ctas = 0;                                           // co-residency limit of k_backsolve_wave on this device
     unsigned long long* bs_cells = nullptr; size_t bs_cells_blocks = 0; // x cells of the wavefront ([block][32][2 words])
     uint32_t bs_epoch = 0;
-    int unblocked_wave = 1;                                             // nb = 1, m <= 8192: the column loop as one persistent launch
-    unsigned int* uw_flags = nullptr; size_t uw_flags_n = 0; unsigned int uw_epoch = 0;
-    int fuse_house = 1;                                                 // nb = 1: next reflector formed inside the apply kernel (one launch per column)
-    int cvy_persist = 1;                                                // 128-wide gemm_cvy: consecutive tiles per CTA (0: one-tile kernel)
-    int cvy_defer = 1;                                                  // 128-wide gemm_cvy: C tile read in batches behind the k-stages
-    int cvy_warps = 8;                                                  // MMA warps per gemm_cvy CTA (4: 64x32 warp tiles, 8: 32x32)
-    int tail_cols = 0;                                                  // trailing width below which the chain is considered critical
-    int wide_panel_ctas = 64;                                           // panel CTAs while the bulk update is wide
-    bool bulk_wide = true;                                              // set per step by the look-ahead driver
-    int panel_ctas_hint = 0;                                            // set per panel by the look-ahead driver (0 = default)
-    int hp_max_ctas = 0;                                                // cap on gemm_vta CTAs of the panel chain under look-ahead (0 = none)
-    long long* panel_trace = nullptr;                                   // optional k_panel clock stamps (option "panel_trace")
+    unsigned int* uw_flags = nullptr; size_t uw_flags_n = 0; unsigned int uw_epoch = 0;   // k_unblocked_wave column flags
     // 128-column panel chain (dhqr_wide.cuh)
     int wide_panel = 1;                                                 // option: factor full aligned outer panels with CholeskyQR2 + reconstruction
     WideCtl* wctl = nullptr;                                            // device control words (first refused panel, guards of the panel in flight)
     double* wbuf = nullptr;                                             // R1, R2, X2, Rt, Y3 (plain 128x128) + XL, XL3 (rmul operand layout)
     int64_t wide_panels = 0, wide_redone = 0;                           // statistics: panels factored by the wide chain / factorisations restarted
     double wide_kappa = 1000.0;                                         // guard on ||D R1^{-1}||_F of the first Cholesky factor (option "wide_kappa")
-    long long* wstamps = nullptr;                                       // clock64 stamps of the single-CTA kernels (option "wide_trace")
-    int wide_trace = 0;
     // Q'b / Qb with one right-hand side: T' of every local panel (computed before the sweep), per-CTA partials of V'b, y, ticket
     double* qt_T = nullptr;  size_t qt_T_elems = 0;
     double* qt_part = nullptr; unsigned int* qt_ticket = nullptr;
-    int gram_sym = 1;                                                   // option: Gram matrices of a packed panel by k_gram_sym (0: k_gemm_vta with the panel as both operands)
     int qt_vec = 1;                                                     // option: use it (0: the GEMM-shaped block update also for one right-hand side)
     double* v1 = nullptr;    size_t v1_elems = 0;                       // unblocked path: v
     double* xbuf = nullptr;  size_t xbuf_elems = 0;                     // back-substitution output
@@ -176,7 +155,7 @@ struct dhqr_context {
     cudaStream_t copy_stream = nullptr;      // compute stream of the _host_ entry points
     cudaStream_t d2h_stream = nullptr;       // drains finished panels to the host while the factorisation continues
     cudaStream_t h2d_stream = nullptr;       // uploads the later column chunks while the first ones are being factored
-    cudaStream_t cu_stream[3] = {nullptr, nullptr, nullptr};   // catch-up: reflectors of finished panels applied to a column chunk that arrived late (chunks alternate)
+    cudaStream_t cu_stream[CU_STREAMS] = {};   // catch-up: reflectors of finished panels applied to a column chunk that arrived late (chunks alternate)
     // dhqr_qr_host_f64 -> look-ahead driver: column chunks still on their way to the device.  Chunk j = global columns [c0, c1),
     // usable once `ev` has fired, joins the trailing matrix at step `join` (after a catch-up with the reflectors of panels < join)
     struct UpChunk { int64_t c0, c1; cudaEvent_t ev; int join; };
@@ -185,7 +164,6 @@ struct dhqr_context {
     int host_first = 0;                      // option: columns of the first upload (0: three panels)
     int host_h2d_gbs = 50, host_tflops = 27; // option: what the join-step planner assumes about the link and the device
     int host_chain_us = 300;                 // option: ... and about the duration of a step of the schedule while the window is narrow
-    int host_cu_streams = 3;                 // option: catch-up streams in use (1..3)
     std::vector<cudaEvent_t> panel_events;
     // set by dhqr_qr_host_f64: finished columns are copied back as soon as their panel is final
     double* mirror_host = nullptr;
@@ -207,7 +185,8 @@ static constexpr int MAXCTAS_FACTOR = 3;
 // gemm tile configurations
 static constexpr int G1_BN = 64, G1_NPW = 2;                // gemm_vta<128>: 128 x 64 tile, 8 MMA + 2 TMA warps
 static constexpr int G1S_BN = 128, G1S_NPW = 4;             // gemm_vta<32> : 32 x 128 tile, 4 MMA + 4 TMA warps
-static constexpr int G2_BM = 128, G2_BN = YT;               // gemm_cvy: 128 x 64 tile, 4 MMA + 1 TMA warps, 2 CTAs/SM
+static constexpr int G2_BM = 128, G2_BN = YT;               // gemm_cvy: 128 x 64 tile, 8 MMA + 1 TMA warps, 2 CTAs/SM
+static constexpr int CVY_TILES_PER_CTA = 1;                 // gemm_cvy_p: tiles one CTA walks through (short-lived CTAs leave SMs to the panel chain)
 
 static size_t smem_g1(int nbp, int bn) { return (size_t)2 * (nbp + bn) * LD1 * 8 + 4 * 8; }
 static size_t smem_g2() { return (size_t)2 * (2 * KC * LD1 + G2_BN * LDK) * 8 + 4 * 8; }
@@ -216,20 +195,13 @@ static size_t smem_ymake(int nbp) { return ((size_t)nbp * nbp + YCOLS * nbp) * 8
 
 #define K_G1_128 k_gemm_vta<128, G1_BN, 4, 2, G1_NPW>
 #define K_G1_32 k_gemm_vta<32, G1S_BN, 1, 4, G1S_NPW>
-#define K_G2 k_gemm_cvy<2, 2, false>
-#define K_G2W k_gemm_cvy<4, 2, false>
-#define K_G2D k_gemm_cvy<4, 2, true>
 
 static int set_attrs(dhqr_context* c) {
     if (c->attrs_set) return 0;
     CU(cudaFuncSetAttribute(K_G1_128, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_g1(128, G1_BN)));
     CU(cudaFuncSetAttribute(K_G1_32, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_g1(32, G1S_BN)));
-    CU(cudaFuncSetAttribute(K_G2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_g2()));
-    CU(cudaFuncSetAttribute(K_G2, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-    CU(cudaFuncSetAttribute(K_G2W, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_g2()));
-    CU(cudaFuncSetAttribute(K_G2W, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
-    CU(cudaFuncSetAttribute(K_G2D, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_g2()));
-    CU(cudaFuncSetAttribute(K_G2D, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
+    CU(cudaFuncSetAttribute(k_gemm_cvy, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_g2()));
+    CU(cudaFuncSetAttribute(k_gemm_cvy, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
     CU(cudaFuncSetAttribute(k_gemm_cvy_p, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_g2()));
     CU(cudaFuncSetAttribute(k_gemm_cvy_p, cudaFuncAttributePreferredSharedMemoryCarveout, 100));
     CU(cudaFuncSetAttribute(k_gram_sym, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM_GRAM_SYM));
@@ -272,10 +244,10 @@ static int ensure_workspace(dhqr_context* c, int64_t m, int64_t n_local_max, int
         for (int b = 0; b < 3; ++b) TRY(ensure(&c->vpk2[b], &c->vpk_elems[b], (size_t)(vrows / KC1) * VPK_CHUNK));
         c->vrows_cap = vrows;
     }
-    if (catchup) for (int b = 3; b < 3 + c->host_cu_streams; ++b) TRY(ensure(&c->vpk2[b], &c->vpk_elems[b], (size_t)(vrows / KC1) * VPK_CHUNK));
+    if (catchup) for (int b = 3; b < 3 + CU_STREAMS; ++b) TRY(ensure(&c->vpk2[b], &c->vpk_elems[b], (size_t)(vrows / KC1) * VPK_CHUNK));
     TRY(ensure(&c->linv_all, &c->linv_all_elems, (size_t)std::max<int64_t>(npanels, 4) * NBMAX * NBMAX));
     const int64_t tiles_max = (n_local_max + NBMAX + G1_BN - 1) / G1_BN + 1;
-    for (int b = 0; b < (catchup ? 3 + c->host_cu_streams : 3); ++b) {
+    for (int b = 0; b < (catchup ? 3 + CU_STREAMS : 3); ++b) {
         auto& w = c->ws[b];
         // set 2 only ever updates the <= 128 columns of one panel: a quarter of the split-K partial buffer is plenty
         TRY(ensure(&w.wpart, &w.wpart_elems, (size_t)(b != 2 ? std::max(WPART_TILES, tiles_max) : WPART_TILES / 4) * NBMAX * G1_BN));
@@ -284,7 +256,6 @@ static int ensure_workspace(dhqr_context* c, int64_t m, int64_t n_local_max, int
         TRY(ensure(&w.linv, &w.linv_elems, (size_t)NBMAX * NBMAX));
     }
     size_t one = 0;
-    if (!c->sm_ticket) { CU(cudaMalloc((void**)&c->sm_ticket, sizeof(unsigned int) * 1024)); CU(cudaMemset(c->sm_ticket, 0, sizeof(unsigned int) * 1024)); }
     if (!c->cells2) {
         const size_t words = (2 * (size_t)(PANEL_MAXG + 1) * (IB * (IB + 1) / 2) + IB * IB + 2 * IB) * 2;
         CU(cudaMalloc((void**)&c->cells2, words * sizeof(unsigned long long)));
@@ -300,8 +271,6 @@ static int ensure_workspace(dhqr_context* c, int64_t m, int64_t n_local_max, int
         CU(cudaMemcpy(c->wctl, &init, sizeof(init), cudaMemcpyHostToDevice));
         size_t o3 = 0;
         TRY(ensure(&c->wbuf, &o3, (size_t)5 * WP * WP + 3 * XL_ELEMS));
-        CU(cudaMalloc((void**)&c->wstamps, 32 * sizeof(long long)));
-        CU(cudaMemset(c->wstamps, 0, 32 * sizeof(long long)));
     }
     TRY(ensure(&c->v1, &c->v1_elems, (size_t)2 * rup(m + 4, 2)));
     TRY(ensure(&c->xbuf, &c->xbuf_elems, (size_t)1));
@@ -347,20 +316,15 @@ static int post(dhqr_context* c, cudaStream_t st, const char* what, double work 
 // block-reflector application  C <- (I - V T' V') C  on window rows >= row_lo
 //   V: nbp columns of the packed V buffer starting at Vcols (window row 0), T from the Gram matrix.
 // ------------------------------------------------------------------------------------------------
-// splits over the row chunks: fill whole waves of SMs; `max_chunks` (> 0) caps the chunks one CTA runs
-// through (look-ahead wants short-lived CTAs so that the high-priority panel chain gets SMs quickly)
-static int pick_splits(int tiles, int nchunks, int sms, int max_chunks, int64_t cap_tiles, int max_ctas = 0) {
+// splits over the row chunks: fill whole waves of SMs
+static int pick_splits(int tiles, int nchunks, int sms, int64_t cap_tiles) {
     tiles = std::max(tiles, 1);
-    int smin = 1;
-    if (max_chunks > 0) smin = std::max(1, (nchunks + max_chunks - 1) / max_chunks);
     int smax = std::max(1, std::min(nchunks / 4, (MAXCTAS_FACTOR * sms) / tiles));
-    smax = std::max(smax, std::min(smin + (sms + tiles - 1) / tiles, std::max(1, nchunks / 2)));
+    smax = std::max(smax, std::min(1 + (sms + tiles - 1) / tiles, std::max(1, nchunks / 2)));
     smax = (int)std::min<int64_t>(smax, std::max<int64_t>(1, cap_tiles / tiles));
-    if (max_ctas > 0) smax = std::min(smax, std::max(1, max_ctas / tiles));
-    smin = std::min(smin, smax);
-    int best = smin;
+    int best = 1;
     double beste = 0.0;
-    for (int s = smin; s <= smax; ++s) {
+    for (int s = 1; s <= smax; ++s) {
         const int ctas = tiles * s;
         const double e = (double)ctas / ((double)sms * ((ctas + sms - 1) / sms));
         if (e > beste + 1e-9) { beste = e; best = s; }
@@ -372,8 +336,8 @@ static int pick_splits(int tiles, int nchunks, int sms, int max_chunks, int64_t 
 //   V = packed columns [voff, voff + nbp) of `vpk` (columns beyond the live ones are zero); T from the
 //   Gram matrix; `w` = the workspace set of the calling chain.
 static int apply_block_reflector(dhqr_context* c, cudaStream_t st, const double* vpk, dhqr_context::WSet& w, int voff, int nbp,
-                                 int64_t rows, int64_t row_lo, double* C, int64_t ldc, int ncols, int max_chunks = 0,
-                                 bool reuse_T = false, double* linv_io = nullptr, int gate = 0, int trans = 0) {
+                                 int64_t rows, int64_t row_lo, double* C, int64_t ldc, int ncols, bool reuse_T = false,
+                                 double* linv_io = nullptr, int gate = 0, int trans = 0) {
     double* linv = linv_io ? linv_io : w.linv;   // where T' is written (or read from, with reuse_T)
     // reuse_T: w.linv already holds T' of this V (same chain, previous call) -> skip the Gram block and k_tinv
     if (ncols <= 0 || rows <= 0) return 0;
@@ -384,8 +348,7 @@ static int apply_block_reflector(dhqr_context* c, cudaStream_t st, const double*
     const int next = nv + ncols;
     const int tiles = (next + bn - 1) / bn;
     const int nchunks = (int)((rows + KC1 - 1) / KC1);
-    const int nsplit = pick_splits(tiles, nchunks, c->sms, max_chunks, (int64_t)(w.wpart_elems / ((size_t)bn * NBPK)),
-                                   (st == c->hp_stream && c->lookahead && c->bulk_wide) ? c->hp_max_ctas : 0);
+    const int nsplit = pick_splits(tiles, nchunks, c->sms, (int64_t)(w.wpart_elems / ((size_t)bn * NBPK)));
     const int64_t pstride = (int64_t)tiles * bn * NBPK;
     if ((size_t)(pstride * nsplit) > w.wpart_elems) return set_err(4001, "internal: W partial workspace too small");
     if ((size_t)next * NBPK > w.wsum_elems) return set_err(4003, "internal: W workspace too small");
@@ -428,16 +391,12 @@ static int apply_block_reflector(dhqr_context* c, cudaStream_t st, const double*
     g2.C = C; g2.ldc = ldc; g2.rows = rows; g2.row_lo = row_lo; g2.ncols = ncols;
     g2.vpk = vpk; g2.voff = voff; g2.ypk = w.ypk;
     g2.nkq = small ? 1 : (int)(rup(nbp, KC) / KC); g2.nkq_alloc = NBPK / KC;
-    g2.sm_ticket = c->cvy_stagger ? c->sm_ticket : nullptr; g2.first_wave = 2 * c->sms; g2.stagger_cycles = 5200 * g2.nkq;
     g2.ctl = c->wctl; g2.gate = gate;
     dim3 grid2((unsigned)((rows + G2_BM - 1) / G2_BM), (unsigned)((ncols + G2_BN - 1) / G2_BN));
     g2.tiles_m = (int)grid2.x; g2.tiles_n = (int)grid2.y;
-    g2.tiles_per_cta = c->cvy_persist;
-    if (c->cvy_warps == 8 && g2.nkq == 4 && c->cvy_persist > 0)
-        k_gemm_cvy_p<<<(g2.tiles_m * g2.tiles_n + c->cvy_persist - 1) / c->cvy_persist, 9 * 32, smem_g2(), st>>>(g2);
-    else if (c->cvy_warps == 8 && g2.nkq == 4 && c->cvy_defer) K_G2D<<<grid2, 9 * 32, smem_g2(), st>>>(g2);
-    else if (c->cvy_warps == 8) K_G2W<<<grid2, 9 * 32, smem_g2(), st>>>(g2);
-    else K_G2<<<grid2, 5 * 32, smem_g2(), st>>>(g2);
+    g2.tiles_per_cta = CVY_TILES_PER_CTA;
+    if (g2.nkq == 4) k_gemm_cvy_p<<<(g2.tiles_m * g2.tiles_n + CVY_TILES_PER_CTA - 1) / CVY_TILES_PER_CTA, 9 * 32, smem_g2(), st>>>(g2);
+    else k_gemm_cvy<<<grid2, 9 * 32, smem_g2(), st>>>(g2);
     TRY(post(c, st, small ? "k_gemm_cvy32" : "k_gemm_cvy128", 2.0 * (double)rows * (small ? 32 : nbp) * (double)ncols));
     return 0;
 }
@@ -447,7 +406,8 @@ static int apply_block_reflector(dhqr_context* c, cudaStream_t st, const double*
 // ------------------------------------------------------------------------------------------------
 static int launch_panel(dhqr_context* c, cudaStream_t st, double* vpk, double* P, int64_t ldp, int64_t mp, int ncols,
                         double* alpha, int voff, int64_t vtop, int64_t vrows, int gate = 0) {
-    int gmax = c->panel_ctas > 0 ? c->panel_ctas : (c->panel_ctas_hint > 0 ? c->panel_ctas_hint : (c->lookahead ? 64 : c->sms));
+    // under look-ahead the panel kernel leaves most SMs to the bulk update running beside it
+    int gmax = c->lookahead ? 64 : c->sms;
     gmax = std::min(std::min(gmax, c->sms), PANEL_MAXG);
     int64_t rpc = std::max<int64_t>((mp + gmax - 1) / gmax, 64);
     rpc = rup(rpc, 8);
@@ -468,7 +428,7 @@ static int launch_panel(dhqr_context* c, cudaStream_t st, double* vpk, double* P
     a.P = P; a.ldp = ldp; a.mp = mp; a.ncols = ncols; a.alpha = alpha;
     a.vpk = vpk; a.voff = voff; a.vtop = vtop; a.vrows = vrows;
     a.rows_per_cta = (int)rpc; a.lds = lds;
-    a.cells = c->cells; a.epoch = c->ll_epoch; a.trace = c->panel_trace; a.backoff = c->panel_backoff; a.levels = c->panel_levels;
+    a.cells = c->cells; a.epoch = c->ll_epoch;
     a.cells2 = c->cells2; a.fast = c->panel_fast; a.fast_stats = c->fast_stats;
     a.ctl = c->wctl; a.gate = gate;
     void* args[] = {&a};
@@ -552,7 +512,7 @@ static int factor_outer_panel_narrow(dhqr_context* c, cudaStream_t st, double* v
         TRY(launch_panel(c, st, vpk, P, lda, m - cs, ib, alpha + cs, o, cs - g.r0, g.vrows, step));
         const int rem = p.kb - (o + ib);
         if (rem > 0)   // update the rest of the outer panel with this sub-panel's reflectors
-            TRY(apply_block_reflector(c, st, vpk, w, o, IB, g.rows, cs - g.r0, A + (cs + ib - col0) * lda + g.r0, lda, rem, 0, false,
+            TRY(apply_block_reflector(c, st, vpk, w, o, IB, g.rows, cs - g.r0, A + (cs + ib - col0) * lda + g.r0, lda, rem, false,
                                       nullptr, step));
     }
     if (g.nbp > IB && g.nbp < NBMAX) {   // zero the V columns the 128-wide kernels read beyond nbp
@@ -567,23 +527,13 @@ static int launch_panel_gram(dhqr_context* c, cudaStream_t st, const double* vpk
                              int64_t* pstride_out) {
     const int nchunks = (int)((rows + KC1 - 1) / KC1);
     const int64_t pstride = (int64_t)WP * WP;
-    int nsplit;
     pre(c, st);
-    if (c->gram_sym) {
-        const int cps = std::max(1, (nchunks + c->sms - 1) / c->sms);                       // chunks per CTA: whole waves of equal CTAs
-        nsplit = (nchunks + cps - 1) / cps;
-        if ((size_t)nsplit * pstride > w.wpart_elems) return set_err(4001, "internal: W partial workspace too small");
-        GramSymArgs g;
-        g.vpk = vpk; g.nchunks = nchunks; g.Wp = w.wpart; g.pstride = pstride;
-        k_gram_sym<<<nsplit, (GS_MMA_WARPS + 1) * 32, SMEM_GRAM_SYM, st>>>(g);
-    } else {
-        const int tiles = WP / G1_BN;
-        nsplit = pick_splits(tiles, nchunks, c->sms, 0, (int64_t)(w.wpart_elems / ((size_t)G1_BN * WP)));
-        GemmVtaArgs g1;
-        g1.vpk = vpk; g1.voff = 0; g1.nv = WP; g1.A = vpk; g1.lda = 2; g1.rows = rows; g1.na = 0; g1.nchunks = nchunks;
-        g1.a_aligned = 1; g1.Wp = w.wpart; g1.pstride = pstride;
-        K_G1_128<<<dim3(tiles, nsplit), (4 * 2 + G1_NPW) * 32, smem_g1(128, G1_BN), st>>>(g1);
-    }
+    const int cps = std::max(1, (nchunks + c->sms - 1) / c->sms);                           // chunks per CTA: whole waves of equal CTAs
+    const int nsplit = (nchunks + cps - 1) / cps;
+    if ((size_t)nsplit * pstride > w.wpart_elems) return set_err(4001, "internal: W partial workspace too small");
+    GramSymArgs g;
+    g.vpk = vpk; g.nchunks = nchunks; g.Wp = w.wpart; g.pstride = pstride;
+    k_gram_sym<<<nsplit, (GS_MMA_WARPS + 1) * 32, SMEM_GRAM_SYM, st>>>(g);
     *nsplit_out = nsplit;
     *pstride_out = pstride;
     return post(c, st, "k_gram128", 2.0 * (double)rows * WP * WP);
@@ -601,7 +551,6 @@ static int factor_outer_panel_wide(dhqr_context* c, cudaStream_t st, double* vpk
     double* Z1 = MT + WP * WP, *Z2 = Z1 + XL_ELEMS, *Z23 = Z2 + XL_ELEMS;
     double* vflag = vpk + KC1;                  // padding row 64 of packed column 0: travels with the V buffer
     const int nq = (int)(g.vrows / KC1);
-    long long* stamps = c->wide_trace ? c->wstamps : nullptr;
     RmulArgs r;
     r.vpk = vpk; r.ctl = c->wctl; r.step = step; r.P = nullptr; r.ldp = lda; r.mp = g.rows;
     auto rmul = [&](int q0, int n, const double* Z, double* Pout) -> int {
@@ -621,20 +570,19 @@ static int factor_outer_panel_wide(dhqr_context* c, cudaStream_t st, double* vpk
     TRY(post(c, st, "k_pack"));
     TRY(gram());
     pre(c, st);
-    if (c->gram_sym) k_wreduce4<<<(WP * WP * 4) / 256, 256, 0, st>>>(w.wpart, pstride, nsplit, (int64_t)WP * WP, w.wsum);
-    else k_wreduce<<<64, 256, 0, st>>>(w.wpart, pstride, nsplit, (int64_t)WP * WP, w.wsum);
+    k_wreduce4<<<(WP * WP * 4) / 256, 256, 0, st>>>(w.wpart, pstride, nsplit, (int64_t)WP * WP, w.wsum);
     TRY(post(c, st, "k_wreduce"));
     pre(c, st);
-    k_chol128<<<1, 512, SMEM_WIDE1, st>>>(w.wsum, R1, Z1, c->wctl, step, vflag, c->wide_kappa, stamps);
+    k_chol128<<<1, 512, SMEM_WIDE1, st>>>(w.wsum, R1, Z1, c->wctl, step, vflag, c->wide_kappa);
     TRY(post(c, st, "k_chol128"));
     TRY(rmul(0, nq, Z1, nullptr));
     TRY(gram());
     pre(c, st);
-    k_gram2_finish<<<c->gram_sym ? 256 : 64, 256, 0, st>>>(w.wpart, pstride, nsplit, w.wsum, R2, Z2, c->wctl, step, vflag);
+    k_gram2_finish<<<256, 256, 0, st>>>(w.wpart, pstride, nsplit, w.wsum, R2, Z2, c->wctl, step, vflag);
     TRY(post(c, st, "k_gram2_finish"));
     // Two small kernels sit beside the chain, not in it (their own high-priority stream, unless the per-launch profile or the
     // debug sync asks for plain stream order): Rt = R2 R1 overlaps the solve of the top chunks, k_trecon the last pass
-    cudaStream_t sx = (c->wide_aux && !c->profile && !c->sync) ? c->aux_stream : st;
+    cudaStream_t sx = (!c->profile && !c->sync) ? c->aux_stream : st;
     if (sx != st) { CU(cudaEventRecord(c->ev_aux[0], st)); CU(cudaStreamWaitEvent(sx, c->ev_aux[0], 0)); }
     pre(c, sx);
     k_trimm128<<<10, 256, SMEM_TRIMM, sx>>>(R2, R1, Rt, c->wctl, step);
@@ -643,7 +591,7 @@ static int factor_outer_panel_wide(dhqr_context* c, cudaStream_t st, double* vpk
     TRY(rmul(0, 2, Z2, nullptr));
     if (sx != st) CU(cudaStreamWaitEvent(st, c->ev_aux[1], 0));
     pre(c, st);
-    k_hr128<<<1, 512, SMEM_WIDE1, st>>>(vpk, Rt, P, lda, alpha + p.c, Rr, MT, c->wctl, step, stamps ? stamps + 16 : nullptr);
+    k_hr128<<<1, 512, SMEM_WIDE1, st>>>(vpk, Rt, P, lda, alpha + p.c, Rr, MT, c->wctl, step);
     TRY(post(c, st, "k_hr128"));
     if (linv_out) {     // T' of the panel from the reconstruction: the owner's next block update needs neither V'V nor k_tinv
         if (sx != st) { CU(cudaEventRecord(c->ev_aux[2], st)); CU(cudaStreamWaitEvent(sx, c->ev_aux[2], 0)); }
@@ -667,7 +615,7 @@ static int factor_outer_panel(dhqr_context* c, cudaStream_t st, double* vpk, dhq
         k_wide_begin<<<1, 32, 0, st>>>(c->wctl, vpk + KC1);
         TRY(post(c, st, "k_wide_begin"));
     }
-    if (wide) return factor_outer_panel_wide(c, st, vpk, w, p, m, col0, A, lda, alpha, step, c->wide_trecon ? linv_out : nullptr);
+    if (wide) return factor_outer_panel_wide(c, st, vpk, w, p, m, col0, A, lda, alpha, step, linv_out);
     return factor_outer_panel_narrow(c, st, vpk, w, p, m, col0, A, lda, alpha, step);
 }
 
@@ -704,7 +652,7 @@ static int qr_blocked_serial(dhqr_context* c, cudaStream_t st, int64_t m, int64_
             const bool wide = plan_wide(c, pl, panels, k, m);
             TRY(factor_outer_panel(c, st, vpk, w, p, m, col0, A, lda, alpha, k, wide, w.linv));
             TRY(mirror_panel_to_host(c, st, p, m, col0, A, lda));
-            haveT = wide && c->wide_trecon;
+            haveT = wide;
         }
         if (c->nranks > 1) {
             // C2 (S:141-143): the owner's reflectors go to every rank, once per panel instead of once per column
@@ -716,7 +664,7 @@ static int qr_blocked_serial(dhqr_context* c, cudaStream_t st, int64_t m, int64_
         // trailing update of the local columns right of the panel (S:198-213 for nb columns at once)
         const int64_t t0 = std::max(p.c + p.kb, col0);
         if (t0 < lend)
-            TRY(apply_block_reflector(c, st, vpk, w, 0, g.nbp, g.rows, p.c - g.r0, A + (t0 - col0) * lda + g.r0, lda, (int)(lend - t0), 0,
+            TRY(apply_block_reflector(c, st, vpk, w, 0, g.nbp, g.rows, p.c - g.r0, A + (t0 - col0) * lda + g.r0, lda, (int)(lend - t0),
                                       haveT, nullptr, k + 1));
     }
     return 0;
@@ -739,14 +687,15 @@ static int qr_blocked_lookahead(dhqr_context* c, cudaStream_t st, int64_t m, int
     cudaStream_t hp = c->hp_stream;
     std::vector<cudaEvent_t> evPanel(K), evNext(K), evBulk(K), evA2(K);
     std::vector<char> haveA2(K, 0);
-    const unsigned evflags = c->la_trace ? cudaEventDefault : cudaEventDisableTiming;
+    // stage timeline of the pipelined host entry (option host_trace; dhqr_qr_host_f64 is the only caller that mirrors to the host)
+    const bool trace = c->host_trace && c->mirror_host;
+    const unsigned evflags = trace ? cudaEventDefault : cudaEventDisableTiming;
     for (int k = K0; k < K; ++k) {
         CU(cudaEventCreateWithFlags(&evA2[k], cudaEventDisableTiming));
         CU(cudaEventCreateWithFlags(&evPanel[k], evflags));
         CU(cudaEventCreateWithFlags(&evNext[k], evflags));
         CU(cudaEventCreateWithFlags(&evBulk[k], evflags));
     }
-    const int maxch = c->vta_max_chunks;   // 0: no cap on the chunks per gemm_vta CTA (short CTAs did not help the chain)
     // local intersection of the global column range [a, b) -> pointer + count
     auto clip = [&](int64_t a, int64_t b, int64_t& lo, int64_t& hi) { lo = std::max(a, col0); hi = std::min(b, lend); return hi > lo; };
     // publish panel k (already factored on its owner into vpk[k%3]) to every rank.  The collectives run on their own stream:
@@ -803,7 +752,7 @@ static int qr_blocked_lookahead(dhqr_context* c, cudaStream_t st, int64_t m, int
             k_pack<<<grid, 256, 0, cu>>>(A + (pq.c - col0) * lda + pq.c, lda, m - pq.c, pq.kb, 1, vpk_cu, 0, pq.c - gq.r0, gq.vrows);
             TRY(post(c, cu, "k_pack"));
             TRY(apply_block_reflector(c, cu, vpk_cu, ws_cu, 0, gq.nbp, gq.rows, pq.c - gq.r0, A + (u.c0 - col0) * lda + gq.r0, lda,
-                                      (int)(u.c1 - u.c0), 0, haveTslot[q] != 0, c->tslot(q), q + 1));
+                                      (int)(u.c1 - u.c0), haveTslot[q] != 0, c->tslot(q), q + 1));
         }
         cudaEventRecord(done, cu);
         return 0;
@@ -821,7 +770,7 @@ static int qr_blocked_lookahead(dhqr_context* c, cudaStream_t st, int64_t m, int
             const bool wide = plan_wide(c, pl, panels, K0, m);
             if ((rc = factor_outer_panel(c, hp, c->vpk2[K0 % 3], c->ws[1], panels[K0], m, col0, A, lda, alpha, K0, wide, c->tslot(K0)))) break;
             if ((rc = mirror_panel_to_host(c, hp, panels[K0], m, col0, A, lda))) break;
-            if (wide && c->wide_trecon) { ownT[K0] = 1; cudaEventRecord(evNext[K0], hp); }
+            if (wide) { ownT[K0] = 1; cudaEventRecord(evNext[K0], hp); }
         }
         if ((rc = publish(K0))) break;
         for (int k = K0; k < K && !rc; ++k) {
@@ -844,14 +793,13 @@ static int qr_blocked_lookahead(dhqr_context* c, cudaStream_t st, int64_t m, int
                     if (cudaEventCreateWithFlags(&done, evflags) != cudaSuccess) { rc = set_err(1001, "event create failed"); break; }
                     evCatch.push_back(done);
                     joinedAt.push_back(k);
-                    if ((rc = catch_up(u, (int)(upnext % (size_t)c->host_cu_streams), k, done))) break;
+                    if ((rc = catch_up(u, (int)(upnext % CU_STREAMS), k, done))) break;
                     wend = u.c1;
                     ++upnext;
                 }
                 if (rc) break;
                 if (wend < t2) { rc = set_err(4005, "internal: window ends at %lld before panel %d", (long long)wend, k + 2); break; }
             }
-            c->bulk_wide = (c->tail_cols <= 0) || (lend - t1 >= c->tail_cols);   // bulk-bound (wide) vs chain-bound (narrow) phase
             double* lk = c->tslot(k);
             bool haveT = ownT[k];                                        // T'_k in lk (this rank)
             if (k + 1 < K) {
@@ -867,19 +815,14 @@ static int qr_blocked_lookahead(dhqr_context* c, cudaStream_t st, int64_t m, int
                     if (clip(t0, t1, lo, hi)) {
                         const bool hadT = haveT;
                         if ((rc = apply_block_reflector(c, hp, vk, c->ws[1], 0, g.nbp, g.rows, p.c - g.r0, A + (lo - col0) * lda + g.r0,
-                                                        lda, (int)(hi - lo), 0, haveT, lk, k + 1))) break;
+                                                        lda, (int)(hi - lo), haveT, lk, k + 1))) break;
                         haveT = true;
                         if (!hadT) cudaEventRecord(evNext[k], hp);       // T'_k is in the ring: the bulk update may start
                     }
-                    // while the bulk update is wide the panel kernel leaves most SMs to it (64 CTAs); once the trailing
-                    // matrix is narrow the chain is the critical path and the panel takes every SM
-                    c->panel_ctas_hint = c->bulk_wide ? c->wide_panel_ctas : (c->tail_cols > 0 ? c->sms : c->wide_panel_ctas);
                     const bool widen = plan_wide(c, pl, panels, k + 1, m);
-                    rc = factor_outer_panel(c, hp, c->vpk2[(k + 1) % 3], c->ws[1], panels[k + 1], m, col0, A, lda, alpha, k + 1, widen,
-                                            c->tslot(k + 1));
-                    c->panel_ctas_hint = 0;
-                    if (rc) break;
-                    if (widen && c->wide_trecon) { ownT[k + 1] = 1; cudaEventRecord(evNext[k + 1], hp); }
+                    if ((rc = factor_outer_panel(c, hp, c->vpk2[(k + 1) % 3], c->ws[1], panels[k + 1], m, col0, A, lda, alpha, k + 1, widen,
+                                                 c->tslot(k + 1)))) break;
+                    if (widen) { ownT[k + 1] = 1; cudaEventRecord(evNext[k + 1], hp); }
                     if ((rc = mirror_panel_to_host(c, hp, panels[k + 1], m, col0, A, lda))) break;
                 }
                 if ((rc = publish(k + 1))) break;
@@ -888,16 +831,14 @@ static int qr_blocked_lookahead(dhqr_context* c, cudaStream_t st, int64_t m, int
             // stream (it overlaps the factorisation of panel k+1); the chain picks it up through evA2[k] before it applies
             // V_{k+1} to the same columns.
             if (clip(t1, t2, lo, hi)) {
-                cudaStream_t s2 = c->hp2 ? c->hp2_stream : hp;
-                if (s2 != hp) {
-                    cudaEventRecord(evA2[k], hp);                        // (used as a scratch event first: order s2 behind hp so far,
-                    cudaStreamWaitEvent(s2, evA2[k], 0);                 //  i.e. behind T'_k and behind the last reader of workspace set 2)
-                }
+                cudaStream_t s2 = c->hp2_stream;
+                cudaEventRecord(evA2[k], hp);                            // (used as a scratch event first: order s2 behind hp so far,
+                cudaStreamWaitEvent(s2, evA2[k], 0);                     //  i.e. behind T'_k and behind the last reader of workspace set 2)
                 if (k - 1 >= K0) cudaStreamWaitEvent(s2, evBulk[k - 1], 0);
                 wait_panel(s2, k);
                 const bool hadT = haveT;
-                if ((rc = apply_block_reflector(c, s2, vk, s2 != hp ? c->ws[2] : c->ws[1], 0, g.nbp, g.rows, p.c - g.r0,
-                                                A + (lo - col0) * lda + g.r0, lda, (int)(hi - lo), 0, haveT, lk, k + 1))) break;
+                if ((rc = apply_block_reflector(c, s2, vk, c->ws[2], 0, g.nbp, g.rows, p.c - g.r0, A + (lo - col0) * lda + g.r0, lda,
+                                                (int)(hi - lo), haveT, lk, k + 1))) break;
                 haveT = true;
                 if (!hadT) cudaEventRecord(evNext[k], s2);               // T'_k came from this apply
                 cudaEventRecord(evA2[k], s2);
@@ -908,47 +849,42 @@ static int qr_blocked_lookahead(dhqr_context* c, cudaStream_t st, int64_t m, int
             if (clip(t2, std::min(lend, wold), lo, hi)) {
                 if (haveT) cudaStreamWaitEvent(st, evNext[k], 0);
                 if ((rc = apply_block_reflector(c, st, vk, c->ws[0], 0, g.nbp, g.rows, p.c - g.r0, A + (lo - col0) * lda + g.r0, lda,
-                                                (int)(hi - lo), maxch, haveT, haveT ? lk : nullptr, k + 1))) break;
+                                                (int)(hi - lo), haveT, haveT ? lk : nullptr, k + 1))) break;
             }
             for (size_t j = up0; j < upnext && !rc; ++j) {             // the chunks that joined at this step, each behind its catch-up
                 const auto& u = c->up_chunks[j];
                 cudaStreamWaitEvent(st, evCatch[j], 0);
                 if (haveT) cudaStreamWaitEvent(st, evNext[k], 0);
                 rc = apply_block_reflector(c, st, vk, c->ws[0], 0, g.nbp, g.rows, p.c - g.r0, A + (u.c0 - col0) * lda + g.r0, lda,
-                                           (int)(u.c1 - u.c0), maxch, haveT, haveT ? lk : nullptr, k + 1);
+                                           (int)(u.c1 - u.c0), haveT, haveT ? lk : nullptr, k + 1);
             }
             if (rc) break;
             haveTslot[k] = haveT;
             cudaEventRecord(evBulk[k], st);
         }
         if (rc) break;
-        c->bulk_wide = true;
         cudaStreamWaitEvent(st, evPanel[K - 1], 0);                // join: alpha and the last panel come from hp / the comm stream
         if (c->nranks > 1) {
             cudaEventRecord(evHp[K - 1], hp);                      // (re-recorded: everything queued on hp)
             cudaStreamWaitEvent(st, evHp[K - 1], 0);
         }
-        if (c->la_trace) {
+        if (trace) {   // ms since the first chunk was on the device
             cudaStreamSynchronize(st);
             cudaStreamSynchronize(hp);
-            c->la_times.assign((size_t)K * 3, 0.f);
-            for (int k = K0; k < K; ++k) {
-                cudaEventElapsedTime(&c->la_times[3 * k + 0], fork, evPanel[k]);
-                cudaEventElapsedTime(&c->la_times[3 * k + 1], fork, evNext[k]);
-                cudaEventElapsedTime(&c->la_times[3 * k + 2], fork, evBulk[k]);
+            for (size_t j = 0; j < evCatch.size(); ++j) {
+                float tu = -1.f, tc = -1.f;
+                cudaEventSynchronize(evCatch[j]);
+                cudaEventElapsedTime(&tu, fork, c->up_chunks[j].ev);
+                cudaEventElapsedTime(&tc, fork, evCatch[j]);
+                fprintf(stderr, "[dhqr host] chunk at column %5lld: uploaded %7.2f ms, joins at step %2d (planned %2d), caught up %7.2f ms\n",
+                        (long long)c->up_chunks[j].c0, tu, joinedAt[j], c->up_chunks[j].join, tc);
             }
-            if (c->host_trace) {   // stage timeline of the pipelined host entry (ms since the first chunk was on the device)
-                for (size_t j = 0; j < evCatch.size(); ++j) {
-                    float tu = -1.f, tc = -1.f;
-                    cudaEventSynchronize(evCatch[j]);
-                    cudaEventElapsedTime(&tu, fork, c->up_chunks[j].ev);
-                    cudaEventElapsedTime(&tc, fork, evCatch[j]);
-                    fprintf(stderr, "[dhqr host] chunk at column %5lld: uploaded %7.2f ms, joins at step %2d (planned %2d), caught up %7.2f ms\n",
-                            (long long)c->up_chunks[j].c0, tu, joinedAt[j], c->up_chunks[j].join, tc);
-                }
-                for (int k = K0; k < K; ++k)
-                    fprintf(stderr, "[dhqr host] step %2d: panel %7.2f  T' %7.2f  bulk %7.2f ms\n", k, c->la_times[3 * k], c->la_times[3 * k + 1],
-                            c->la_times[3 * k + 2]);
+            for (int k = K0; k < K; ++k) {
+                float tp = 0.f, tt = 0.f, tb = 0.f;
+                cudaEventElapsedTime(&tp, fork, evPanel[k]);
+                cudaEventElapsedTime(&tt, fork, evNext[k]);
+                cudaEventElapsedTime(&tb, fork, evBulk[k]);
+                fprintf(stderr, "[dhqr host] step %2d: panel %7.2f  T' %7.2f  bulk %7.2f ms\n", k, tp, tt, tb);
             }
         }
     } while (0);
@@ -960,7 +896,7 @@ static int qr_blocked_lookahead(dhqr_context* c, cudaStream_t st, int64_t m, int
         cudaStreamWaitEvent(st, hpdone, 0);
         cudaEventRecord(hpdone, c->hp2_stream);
         cudaStreamWaitEvent(st, hpdone, 0);
-        for (int i = 0; i < 3; ++i) {
+        for (int i = 0; i < CU_STREAMS; ++i) {
             cudaEventRecord(hpdone, c->cu_stream[i]);
             cudaStreamWaitEvent(st, hpdone, 0);
         }
@@ -1041,7 +977,7 @@ static int qr_unblocked(dhqr_context* c, cudaStream_t st, int64_t m, int64_t n, 
     TRY(check_partition(col0s, nls, n));
     TRY(ensure_workspace(c, m, nl));
     const int64_t lend = col0 + nl;
-    if (c->nranks == 1 && n > 0 && m <= (int64_t)UW_MAXI * UW_THREADS && c->unblocked_wave && !c->profile && !c->sync) {
+    if (c->nranks == 1 && n > 0 && m <= (int64_t)UW_MAXI * UW_THREADS && !c->profile && !c->sync) {
         // single GPU, short columns: the whole column loop as one persistent cooperative launch (k_unblocked_wave)
         if (c->uw_flags_n < (size_t)n) {
             if (c->uw_flags) CU(cudaFree(c->uw_flags));
@@ -1061,7 +997,7 @@ static int qr_unblocked(dhqr_context* c, cudaStream_t st, int64_t m, int64_t n, 
         if (e != cudaSuccess) return set_err(1000 + (int)e, "cooperative launch of k_unblocked_wave failed: %s", cudaGetErrorString(e));
         return post(c, st, "k_unblocked_wave", 16.0 * (double)m * n * n / 2);
     }
-    if (c->nranks == 1 && n > 0 && (size_t)((m + 2) & ~(int64_t)1) * 8 * (A1_CW + 1) <= 200 * 1024 && c->fuse_house) {
+    if (c->nranks == 1 && n > 0 && (size_t)((m + 2) & ~(int64_t)1) * 8 * (A1_CW + 1) <= 200 * 1024) {
         // single GPU, the column tile fits in shared memory: one launch per column step (the next reflector is formed by the
         // CTA that has just updated its column, k_apply1_tma), two v buffers alternating between steps
         const int64_t voff = rup(m + 4, 2);
@@ -1144,7 +1080,7 @@ static int apply_qt_local(dhqr_context* c, cudaStream_t st, int64_t m, int64_t c
         dim3 grid((unsigned)std::min<int64_t>((vrows / 4 + 255) / 256, 4 * c->sms), nbp);
         k_pack<<<grid, 256, 0, st>>>(A + o * lda + cs, lda, m - cs, kb, 1, c->vpk2[0], 0, cs - r0, vrows);
         TRY(post(c, st, "k_pack"));
-        TRY(apply_block_reflector(c, st, c->vpk2[0], c->ws[0], 0, nbp, rows, cs - r0, b + r0, ldb, nrhs, 0, false, nullptr, 0, notrans));
+        TRY(apply_block_reflector(c, st, c->vpk2[0], c->ws[0], 0, nbp, rows, cs - r0, b + r0, ldb, nrhs, false, nullptr, 0, notrans));
     }
     return 0;
 }
@@ -1215,7 +1151,7 @@ static int backsolve_local(dhqr_context* c, cudaStream_t st, int64_t col0, int64
     if (nl <= 0) return 0;
     // one launch per right-hand side: a wavefront over 32-row strips (k_backsolve_wave); needs every CTA resident at once
     const int64_t nbk = (nl + 31) / 32, nlow = (col0 + 31) / 32;
-    if (c->bs_wave && nbk + nlow <= c->bs_wave_max_ctas && nbk <= (int64_t)c->bs_cells_blocks) {
+    if (nbk + nlow <= c->bs_wave_max_ctas && nbk <= (int64_t)c->bs_cells_blocks) {
         for (int rhs = 0; rhs < nrhs; ++rhs) {
             if (c->bs_epoch > 0xFFFFFFF0u) {
                 CU(cudaMemsetAsync(c->bs_cells, 0, (size_t)c->bs_cells_blocks * 32 * 16, st));
@@ -1258,22 +1194,19 @@ static int create_common(dhqr_handle* h, int device) {
     dhqr_context* c = new dhqr_context();
     c->device = device;
     c->sms = prop.multiProcessorCount;
-    if (const char* e = getenv("DHQR_GRAM_SYM")) c->gram_sym = atoi(e) ? 1 : 0;   // A/B runs of whole test suites (tools/)
     CU(cudaMalloc((void**)&c->d_i64, sizeof(int64_t) * 2 * 1025));
     CU(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
     CU(cudaStreamCreateWithFlags(&c->d2h_stream, cudaStreamNonBlocking));
     CU(cudaStreamCreateWithFlags(&c->h2d_stream, cudaStreamNonBlocking));
-    for (int i = 0; i < 3; ++i) CU(cudaStreamCreateWithFlags(&c->cu_stream[i], cudaStreamNonBlocking));
+    for (int i = 0; i < CU_STREAMS; ++i) CU(cudaStreamCreateWithFlags(&c->cu_stream[i], cudaStreamNonBlocking));
     {
         int lo = 0, hi = 0;
         CU(cudaDeviceGetStreamPriorityRange(&lo, &hi));
-        CU(cudaStreamCreateWithPriority(&c->hp_hi, cudaStreamNonBlocking, hi));
-        CU(cudaStreamCreateWithPriority(&c->hp_lo, cudaStreamNonBlocking, lo));
+        CU(cudaStreamCreateWithPriority(&c->hp_stream, cudaStreamNonBlocking, hi));
         CU(cudaStreamCreateWithPriority(&c->comm_stream, cudaStreamNonBlocking, hi));
         CU(cudaStreamCreateWithPriority(&c->hp2_stream, cudaStreamNonBlocking, hi));
         CU(cudaStreamCreateWithPriority(&c->aux_stream, cudaStreamNonBlocking, hi));
         for (int i = 0; i < 4; ++i) CU(cudaEventCreateWithFlags(&c->ev_aux[i], cudaEventDisableTiming));
-        c->hp_stream = c->hp_hi;
     }
     *h = c;
     return 0;
@@ -1313,16 +1246,15 @@ int dhqr_destroy(dhqr_handle c) {
     cudaDeviceSynchronize();
     if (c->comm) g_nccl.CommDestroy(c->comm);
     cudaFree(c->linv_all);
-    for (int b = 0; b < 6; ++b) {
+    for (int b = 0; b < 3 + CU_STREAMS; ++b) {
         cudaFree(c->vpk2[b]);
         cudaFree(c->ws[b].wpart); cudaFree(c->ws[b].wsum); cudaFree(c->ws[b].ypk); cudaFree(c->ws[b].linv);
     }
     cudaFree(c->uw_flags);
     cudaFree(c->qt_T); cudaFree(c->qt_part); cudaFree(c->qt_ticket);
-    cudaFree(c->wctl); cudaFree(c->wbuf); cudaFree(c->wstamps); cudaFree(c->bs_cells);
-    cudaFree(c->cells); cudaFree(c->cells2); cudaFree(c->fast_stats); cudaFree(c->panel_trace); cudaFree(c->sm_ticket);
-    if (c->hp_hi) cudaStreamDestroy(c->hp_hi);
-    if (c->hp_lo) cudaStreamDestroy(c->hp_lo);
+    cudaFree(c->wctl); cudaFree(c->wbuf); cudaFree(c->bs_cells);
+    cudaFree(c->cells); cudaFree(c->cells2); cudaFree(c->fast_stats);
+    if (c->hp_stream) cudaStreamDestroy(c->hp_stream);
     if (c->comm_stream) cudaStreamDestroy(c->comm_stream);
     if (c->hp2_stream) cudaStreamDestroy(c->hp2_stream);
     if (c->aux_stream) cudaStreamDestroy(c->aux_stream);
@@ -1332,7 +1264,7 @@ int dhqr_destroy(dhqr_handle c) {
     if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
     if (c->d2h_stream) cudaStreamDestroy(c->d2h_stream);
     if (c->h2d_stream) cudaStreamDestroy(c->h2d_stream);
-    for (int i = 0; i < 3; ++i) if (c->cu_stream[i]) cudaStreamDestroy(c->cu_stream[i]);
+    for (int i = 0; i < CU_STREAMS; ++i) if (c->cu_stream[i]) cudaStreamDestroy(c->cu_stream[i]);
     delete c;
     return 0;
 }
@@ -1343,30 +1275,12 @@ int dhqr_set_option(dhqr_handle c, const char* key, int64_t value) {
     if (!strcmp(key, "nb")) {
         if (value < 32 || value > 128 || value % 32) return set_err(-3, "nb must be a multiple of 32 in [32,128]");
         c->nb = (int)value;
-    } else if (!strcmp(key, "panel_ctas")) {
-        if (value < 0) return set_err(-3, "panel_ctas < 0");
-        c->panel_ctas = (int)value;
     } else if (!strcmp(key, "sync")) {
         c->sync = value ? 1 : 0;
     } else if (!strcmp(key, "profile")) {
         c->profile = value ? 1 : 0;
     } else if (!strcmp(key, "lookahead")) {
         c->lookahead = value ? 1 : 0;
-    } else if (!strcmp(key, "cvy_warps")) {
-        if (value != 4 && value != 8) return set_err(-3, "cvy_warps must be 4 or 8");
-        c->cvy_warps = (int)value;
-    } else if (!strcmp(key, "wide_panel_ctas")) {
-        c->wide_panel_ctas = (int)value;
-    } else if (!strcmp(key, "tail_cols")) {
-        c->tail_cols = (int)value;
-    } else if (!strcmp(key, "hp_priority")) {
-        c->hp_stream = value ? c->hp_hi : c->hp_lo;
-    } else if (!strcmp(key, "hp_max_ctas")) {
-        c->hp_max_ctas = (int)value;
-    } else if (!strcmp(key, "wide_aux")) {
-        c->wide_aux = value ? 1 : 0;
-    } else if (!strcmp(key, "wide_trecon")) {
-        c->wide_trecon = value ? 1 : 0;
     } else if (!strcmp(key, "host_trace")) {
         c->host_trace = value ? 1 : 0;
     } else if (!strcmp(key, "host_chunk")) {
@@ -1381,35 +1295,11 @@ int dhqr_set_option(dhqr_handle c, const char* key, int64_t value) {
     } else if (!strcmp(key, "host_chain_us")) {
         if (value < 1) return set_err(-3, "host_chain_us < 1");
         c->host_chain_us = (int)value;
-    } else if (!strcmp(key, "host_cu_streams")) {
-        if (value < 1 || value > 3) return set_err(-3, "host_cu_streams must be 1, 2 or 3");
-        c->host_cu_streams = (int)value;
     } else if (!strcmp(key, "host_tflops")) {
         if (value < 1) return set_err(-3, "host_tflops < 1");
         c->host_tflops = (int)value;
-    } else if (!strcmp(key, "gram_sym")) {
-        c->gram_sym = value ? 1 : 0;
     } else if (!strcmp(key, "qt_vec")) {
         c->qt_vec = value ? 1 : 0;
-    } else if (!strcmp(key, "hp2")) {
-        c->hp2 = value ? 1 : 0;
-    } else if (!strcmp(key, "bs_wave")) {
-        c->bs_wave = value ? 1 : 0;
-    } else if (!strcmp(key, "unblocked_wave")) {
-        c->unblocked_wave = value ? 1 : 0;
-    } else if (!strcmp(key, "fuse_house")) {
-        c->fuse_house = value ? 1 : 0;
-    } else if (!strcmp(key, "cvy_persist")) {
-        if (value < 0 || value > 1 << 20) return set_err(-3, "cvy_persist out of range");
-        c->cvy_persist = (int)value;
-    } else if (!strcmp(key, "cvy_defer")) {
-        c->cvy_defer = value ? 1 : 0;
-    } else if (!strcmp(key, "cvy_stagger")) {
-        c->cvy_stagger = value ? 1 : 0;
-    } else if (!strcmp(key, "la_trace")) {
-        c->la_trace = value ? 1 : 0;
-    } else if (!strcmp(key, "vta_max_chunks")) {
-        c->vta_max_chunks = (int)value;
     } else if (!strcmp(key, "panel_fast")) {
         c->panel_fast = value ? 1 : 0;
     } else if (!strcmp(key, "wide_panel")) {
@@ -1417,21 +1307,6 @@ int dhqr_set_option(dhqr_handle c, const char* key, int64_t value) {
     } else if (!strcmp(key, "wide_kappa")) {
         if (value < 1) return set_err(-3, "wide_kappa < 1");
         c->wide_kappa = (double)value;
-    } else if (!strcmp(key, "wide_trace")) {
-        c->wide_trace = value ? 1 : 0;
-    } else if (!strcmp(key, "panel_levels")) {
-        if (value != 1 && value != 2) return set_err(-3, "panel_levels must be 1 or 2");
-        c->panel_levels = (int)value;
-    } else if (!strcmp(key, "panel_backoff")) {
-        c->panel_backoff = (int)value;
-    } else if (!strcmp(key, "panel_trace")) {
-        if (value && !c->panel_trace) {
-            CU(cudaMalloc((void**)&c->panel_trace, sizeof(long long) * (size_t)PANEL_MAXG * IB * 8));
-            CU(cudaMemset(c->panel_trace, 0, sizeof(long long) * (size_t)PANEL_MAXG * IB * 8));
-        } else if (!value && c->panel_trace) {
-            CU(cudaFree(c->panel_trace));
-            c->panel_trace = nullptr;
-        }
     } else {
         return set_err(-2, "unknown option '%s'", key);
     }
@@ -1443,15 +1318,21 @@ int dhqr_get_option(dhqr_handle c, const char* key, int64_t* value) {
     if (!key) return set_err(-2, "null key");
     if (!value) return set_err(-3, "null value");
     if (!strcmp(key, "nb")) *value = c->nb;
-    else if (!strcmp(key, "panel_ctas")) *value = c->panel_ctas;
+    else if (!strcmp(key, "lookahead")) *value = c->lookahead;
+    else if (!strcmp(key, "wide_panel")) *value = c->wide_panel;
+    else if (!strcmp(key, "wide_kappa")) *value = (int64_t)c->wide_kappa;
+    else if (!strcmp(key, "panel_fast")) *value = c->panel_fast;
+    else if (!strcmp(key, "qt_vec")) *value = c->qt_vec;
+    else if (!strcmp(key, "host_chunk")) *value = c->host_chunk;
+    else if (!strcmp(key, "host_first")) *value = c->host_first;
+    else if (!strcmp(key, "host_h2d_gbs")) *value = c->host_h2d_gbs;
+    else if (!strcmp(key, "host_tflops")) *value = c->host_tflops;
+    else if (!strcmp(key, "host_chain_us")) *value = c->host_chain_us;
+    else if (!strcmp(key, "host_trace")) *value = c->host_trace;
     else if (!strcmp(key, "sync")) *value = c->sync;
     else if (!strcmp(key, "profile")) *value = c->profile;
-    else if (!strcmp(key, "lookahead")) *value = c->lookahead;
-    else if (!strcmp(key, "panel_fast")) *value = c->panel_fast;
-    else if (!strcmp(key, "wide_panel")) *value = c->wide_panel;
     else if (!strcmp(key, "wide_panels")) *value = c->wide_panels;
     else if (!strcmp(key, "wide_redone")) *value = c->wide_redone;
-    else if (!strcmp(key, "panel_variant")) *value = PANEL_VARIANT;
     else if (!strcmp(key, "panels_fast") || !strcmp(key, "panels_fallback")) {
         int st2[2] = {0, 0};
         if (c->fast_stats) CU(cudaMemcpy(st2, c->fast_stats, sizeof(st2), cudaMemcpyDeviceToHost));
@@ -1859,10 +1740,7 @@ int dhqr_qr_host_f64(dhqr_handle c, int64_t m, int64_t n, double* hA, int64_t ld
         }
         stamp("first chunk uploaded", true);
         if (blocked) { c->mirror_host = hA; c->mirror_lda = lda; }   // finished panels stream back while later panels are factored
-        const int la_trace_keep = c->la_trace;
-        if (c->host_trace) c->la_trace = 1;
         rc = dhqr_qr_f64(c, m, n, 0, n, dA, ldd, dal, nb, st);
-        c->la_trace = la_trace_keep;
         c->mirror_host = nullptr;
         if (rc) break;
         stamp("factored", true);
@@ -1874,7 +1752,7 @@ int dhqr_qr_host_f64(dhqr_handle c, int64_t m, int64_t n, double* hA, int64_t ld
     c->up_chunks.clear();
     cudaError_t e0 = cudaStreamSynchronize(c->h2d_stream), e1 = cudaStreamSynchronize(st), e2 = cudaStreamSynchronize(c->d2h_stream);
     cudaError_t e3 = cudaSuccess;
-    for (int i = 0; i < 3; ++i) { const cudaError_t e4 = cudaStreamSynchronize(c->cu_stream[i]); if (e3 == cudaSuccess) e3 = e4; }
+    for (int i = 0; i < CU_STREAMS; ++i) { const cudaError_t e4 = cudaStreamSynchronize(c->cu_stream[i]); if (e3 == cudaSuccess) e3 = e4; }
     stamp("everything back on the host", false);
     for (cudaEvent_t ev : c->panel_events) cudaEventDestroy(ev);
     c->panel_events.clear();
@@ -1967,12 +1845,6 @@ int dhqr_debug_copy_f64(dhqr_handle c, const char* which, double* d_dst, int64_t
     if (!c) return set_err(-1, "null handle");
     if (!which) return set_err(-2, "null name");
     if (!d_dst) return set_err(-3, "null destination");
-    if (!strcmp(which, "la_times")) {   // host-side list: converted to doubles and copied to the device buffer
-        std::vector<double> t(c->la_times.begin(), c->la_times.end());
-        if ((size_t)nelems < t.size()) return set_err(-4, "need %zu elements", t.size());
-        CU(cudaMemcpy(d_dst, t.data(), t.size() * sizeof(double), cudaMemcpyHostToDevice));
-        return 0;
-    }
     const double* src = nullptr;
     size_t have = 0;
     if (!strcmp(which, "wpart")) { src = c->ws[0].wpart; have = c->ws[0].wpart_elems; }
@@ -1980,9 +1852,7 @@ int dhqr_debug_copy_f64(dhqr_handle c, const char* which, double* d_dst, int64_t
     else if (!strcmp(which, "ypk")) { src = c->ws[0].ypk; have = c->ws[0].ypk_elems; }
     else if (!strcmp(which, "linv")) { src = c->ws[0].linv; have = (size_t)NBMAX * NBMAX; }
     else if (!strcmp(which, "vpk")) { src = c->vpk2[0]; have = c->vpk_elems[0]; }
-    else if (!strcmp(which, "wstamps")) { src = (const double*)c->wstamps; have = c->wstamps ? 32 : 0; }
     else if (!strcmp(which, "wide")) { src = c->wbuf; have = c->wbuf ? (size_t)5 * WP * WP + 3 * XL_ELEMS : 0; }
-    else if (!strcmp(which, "panel_trace")) { src = (const double*)c->panel_trace; have = c->panel_trace ? (size_t)PANEL_MAXG * IB * 8 : 0; }
     else return set_err(-2, "unknown buffer '%s'", which);
     if (nelems < 0 || (size_t)nelems > have) return set_err(-4, "nelems out of range (have %zu)", have);
     CU(cudaMemcpyAsync(d_dst, src, sizeof(double) * (size_t)nelems, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));

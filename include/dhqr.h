@@ -68,25 +68,22 @@ int dhqr_destroy(dhqr_handle h);
  *   "wide_panel"  1 (default): full, 32-aligned outer panels of width 128 are factored by the 128-column chain
  *                 (CholeskyQR2 + Householder reconstruction on the whole panel: 3 grid-wide reductions per 128 columns,
  *                 no cooperative launch); refused panels and all other panels use the 32-column chain below
+ *   "wide_kappa"  guard of the 128-column chain (default 1000, >= 1): a panel whose first Cholesky factor has
+ *                 ||D R1^{-1}||_F above it is refused and redone by the 32-column chain
  *   "panel_fast"  1 (default): inner panels by CholeskyQR2 + Householder reconstruction with on-device fallback
  *                 to the column-by-column kernel; 0: always column by column
- *   "panel_ctas"  CTAs of the cooperative panel kernel (0 = default: 64 under look-ahead, one per SM otherwise)
- *   "cvy_warps"   MMA warps per gemm_cvy CTA: 8 (default, 32x32 warp tiles) or 4 (64x32)
- *   "gram_sym"    1 (default): Gram matrices of a packed 128-column panel by k_gram_sym (chunk staged once, upper blocks only);
- *                 0: k_gemm_vta with the panel as both operands.  Environment DHQR_GRAM_SYM overrides the default at handle creation
  *   "qt_vec"      1 (default): Q'b / Qb with ONE right-hand side as a GEMV sweep (T' of every panel computed first, then two
  *                 HBM-bound launches per panel that read the reflectors in place); 0: the GEMM-shaped block update, as for nrhs > 1
  *   "host_chunk"  columns per upload chunk of dhqr_qr_host_f64 (default 512, a multiple of 128; 0: one upload, no overlap);
  *                 "host_h2d_gbs" (50), "host_tflops" (27), "host_chain_us" (300): what its join-step planner assumes about the
- *                 host link, the device and a step of the schedule on a narrow window; "host_cu_streams" (3): catch-up streams; "host_first" (0 = three panels): columns of the first, exposed upload;
- *                 "host_trace" 1: stage timeline on stderr.  A wrong assumption costs idle time, never correctness
+ *                 host link, the device and a step of the schedule on a narrow window; "host_first" (0 = three panels): columns
+ *                 of the first, exposed upload; "host_trace" 1: stage timeline on stderr.  A wrong assumption costs idle time,
+ *                 never correctness
  *   "sync"        1: cudaStreamSynchronize + error check after every kernel launch (debugging; implies serial)
  *   "profile"     1: CUDA-event bracket per launch (implies serial), read with dhqr_profile_get
  *   read-only:    "sms", "rank", "nranks", "panels_fast", "panels_fallback" (inner panels taken by either path),
- *                 "wide_panels" (outer panels factored by the 128-column chain), "wide_redone" (restarts after a refusal),
- *                 "panel_variant" (compile-time DHQR_PANEL_VARIANT of the panel kernel's fast path)
- *   experiment knobs kept for tools/: "panel_levels", "panel_backoff", "panel_trace", "la_trace", "vta_max_chunks",
- *                 "hp_max_ctas", "hp_priority", "cvy_stagger" */
+ *                 "wide_panels" (outer panels factored by the 128-column chain), "wide_redone" (restarts after a refusal)
+ * Any other key is refused with -2. */
 int dhqr_set_option(dhqr_handle h, const char *key, int64_t value);
 int dhqr_get_option(dhqr_handle h, const char *key, int64_t *value);
 /* Number of kernel launches enqueued by this handle since creation (bench.py: gpu_launches). */

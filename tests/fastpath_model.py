@@ -11,7 +11,7 @@ diagonal blocks, products R_ab inv(R_bb) formed once.
 import numpy as np
 
 IB = 32
-SPREAD_MIN = 4e-3     # FAST_SPREAD_MIN of the kernel for the tensor-pipe solves (1e-5 with row-by-row substitution)
+SPREAD_MIN = 4e-3     # FAST_SPREAD_MIN of the kernel (its triangular solves run on the tensor pipe)
 
 
 def blocked_trsm(X, R, dgi):

@@ -61,7 +61,7 @@ def test_every_panel_the_guards_accept_is_backward_stable(oracle):
 
 
 def test_substitution_guard_would_not_be_enough_for_blocked_solves(oracle, monkeypatch):
-    # documents why the guard differs between the two solve variants: with the substitution guard (spread < 1e5) the blocked
+    # documents why the guard is tighter than row-by-row substitution would need: with a spread up to 1e5 the blocked
     # solves would accept a panel whose factorisation residual is ~1e-13
     monkeypatch.setattr(F, "SPREAD_MIN", 1e-5)
     P = oracle.np_uniform(31, 2048, 32)

@@ -276,6 +276,30 @@ def test_lookahead_and_serial_schedules_agree(D, dev, oracle):
         assert oracle.qr_residual(A0, np.asfortranarray(res[la][0]), res[la][1]) < TOL_RES
 
 
+# Every settable option with its default; anything else is not an option of the library.
+OPTION_DEFAULTS = {"nb": 128, "lookahead": 1, "wide_panel": 1, "wide_kappa": 1000, "panel_fast": 1, "qt_vec": 1,
+                   "host_chunk": 512, "host_first": 0, "host_h2d_gbs": 50, "host_tflops": 27, "host_chain_us": 300,
+                   "host_trace": 0, "sync": 0, "profile": 0}
+RETIRED_OPTIONS = ["cvy_warps", "cvy_persist", "cvy_defer", "cvy_stagger", "hp_priority", "hp_max_ctas", "vta_max_chunks",
+                   "tail_cols", "wide_panel_ctas", "panel_ctas", "wide_aux", "wide_trecon", "hp2", "gram_sym", "bs_wave",
+                   "unblocked_wave", "fuse_house", "panel_levels", "panel_backoff", "panel_trace", "wide_trace", "la_trace",
+                   "host_cu_streams", "panel_variant"]
+
+
+@pytest.mark.parametrize("key", sorted(OPTION_DEFAULTS) + RETIRED_OPTIONS)
+def test_option_keys(D, key):
+    # a documented option takes its default and reads it back; a retired one is an unknown key (-2) both ways
+    h = D.default_handle(0)
+    if key in OPTION_DEFAULTS:
+        h.set_option(key, OPTION_DEFAULTS[key])
+        assert h.get_option(key) == OPTION_DEFAULTS[key]
+        return
+    for op in (lambda: h.set_option(key, 0), lambda: h.get_option(key)):
+        with pytest.raises(D._lib.DhqrError) as e:
+            op()
+        assert e.value.code == -2
+
+
 def test_block_reflector_kernels(D, dev, oracle):
     # gemm_vta + tinv + ymake + gemm_cvy in isolation against torch fp64 on genuine Householder blocks
     h = D.default_handle(0)

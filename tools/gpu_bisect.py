@@ -6,10 +6,8 @@ import torch
 import dhqr_b200 as D
 dev = torch.device("cuda:0")
 h = D.default_handle(0)
-def run(m, n, sync, nb=0, opts=None):
+def run(m, n, sync, nb=0):
     h.set_option("sync", sync)
-    for k, v in (opts or {}).items():
-        h.set_option(k, v)
     A = D.colmajor_empty(m, n, dev); D.fill_uniform_(A, 0)
     al = torch.zeros(n, dtype=torch.float64, device=dev)
     D.householder_(A, al, nb)
@@ -46,5 +44,3 @@ for (m, n) in [(16384, 2048), (32768, 4096)]:
     cmp("sync0 vs sync0", S0, S0b, n)
     S1b = run(m, n, 1)
     cmp("sync1 vs sync1", S1, S1b, n)
-    P = run(m, n, 0, opts={"panel_ctas": 64}); h.set_option("panel_ctas", 0)
-    print(f"{m}x{n} panel_ctas=64 sync=0 resid {resid(*P, m, n):.3e}", flush=True)

@@ -1,5 +1,5 @@
 """dhqr_qr_host_f64 at BASELINE config 3: does it matter who wrote the pinned host buffer last (CPU memcpy as in bench.py's e2e leg vs a
-device-to-host copy as in tools/r3_plans*.py)?  Wall time + upload timeline for both, first upload of 384 / 768 columns."""
+device-to-host copy)?  Wall time + upload timeline for both, first upload of 384 / 768 columns."""
 import os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import ctypes as C
