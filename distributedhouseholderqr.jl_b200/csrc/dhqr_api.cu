@@ -12,6 +12,8 @@
 #include <time.h>
 
 #include <algorithm>
+#include <memory>
+#include <utility>
 #include <vector>
 
 #include "dhqr_kernels.cuh"
@@ -102,6 +104,58 @@ static inline int64_t rup(int64_t x, int64_t a) { return (x + a - 1) / a * a; }
 
 static constexpr int CU_STREAMS = 3;   // catch-up streams of dhqr_qr_host_f64, each with its own V buffer and workspace set
 
+// Owners of the handle's CUDA resources: each releases what it holds when it goes, so neither a failed call nor
+// dhqr_destroy has to know the list of buffers, streams and events.
+template <typename T>
+class DevBuf {   // one zero-filled cudaMalloc allocation and its element count
+  public:
+    DevBuf() = default;
+    DevBuf(DevBuf&& o) noexcept : p_(o.p_), n_(o.n_) { o.p_ = nullptr; o.n_ = 0; }
+    ~DevBuf() { if (p_) cudaFree(p_); }
+    operator T*() const { return p_; }
+    size_t size() const { return n_; }
+    // at least `need` elements: a smaller allocation is freed first and replaced by a zero-filled one of exactly `need`;
+    // *grown says whether that happened
+    int grow(size_t need, bool* grown = nullptr) {
+        if (grown) *grown = false;
+        if (n_ >= need && p_) return 0;
+        if (p_) CU(cudaFree(p_));
+        p_ = nullptr;
+        n_ = 0;
+        CU(cudaMalloc((void**)&p_, need * sizeof(T)));
+        CU(cudaMemset(p_, 0, need * sizeof(T)));
+        n_ = need;
+        if (grown) *grown = true;
+        return 0;
+    }
+  private:
+    T* p_ = nullptr;
+    size_t n_ = 0;
+};
+class Stream {   // a non-blocking stream
+  public:
+    Stream() = default;
+    Stream(const Stream&) = delete;
+    Stream& operator=(const Stream&) = delete;
+    ~Stream() { if (s_) cudaStreamDestroy(s_); }
+    operator cudaStream_t() const { return s_; }
+    cudaError_t create() { return cudaStreamCreateWithFlags(&s_, cudaStreamNonBlocking); }
+    cudaError_t create(int priority) { return cudaStreamCreateWithPriority(&s_, cudaStreamNonBlocking, priority); }
+  private:
+    cudaStream_t s_ = nullptr;
+};
+class Event {   // may go as soon as the work it orders is enqueued; a std::vector<Event> is the event list of one call
+  public:
+    Event() = default;
+    Event(Event&& o) noexcept : e_(o.e_) { o.e_ = nullptr; }
+    Event& operator=(Event&& o) noexcept { std::swap(e_, o.e_); return *this; }
+    ~Event() { if (e_) cudaEventDestroy(e_); }
+    operator cudaEvent_t() const { return e_; }
+    cudaError_t create(unsigned flags) { *this = Event(); return cudaEventCreateWithFlags(&e_, flags); }
+  private:
+    cudaEvent_t e_ = nullptr;
+};
+
 struct dhqr_context {
     int device = 0, sms = 0;
     int rank = 0, nranks = 1;
@@ -111,51 +165,51 @@ struct dhqr_context {
     // workspace
     // three V buffers (panels k, k+1 and the one being broadcast live at the same time under look-ahead) and two
     // workspace sets (set 0: trailing update on the caller's stream; set 1: panel chain on the high-priority stream)
-    double* vpk2[3 + CU_STREAMS] = {}; size_t vpk_elems[3 + CU_STREAMS] = {}; int64_t vrows_cap = 0;   // packed V [chunk][128][68]; [3..]: catch-up of late column chunks (host entry)
+    DevBuf<double> vpk2[3 + CU_STREAMS];                                // packed V [chunk][128][68]; [3..]: catch-up of late column chunks (host entry)
     struct WSet {
-        double* wpart = nullptr; size_t wpart_elems = 0;                // gemm_vta partials
-        double* wsum = nullptr;  size_t wsum_elems = 0;                 // reduced Wext
-        double* ypk = nullptr;   size_t ypk_elems = 0;                  // packed Y = -T'W
-        double* linv = nullptr;  size_t linv_elems = 0;                 // [128*128]
+        DevBuf<double> wpart;                                           // gemm_vta partials
+        DevBuf<double> wsum;                                            // reduced Wext
+        DevBuf<double> ypk;                                             // packed Y = -T'W
+        DevBuf<double> linv;                                            // [128*128]
     } ws[3 + CU_STREAMS];                                               // [2]: the chain's second apply (columns of panel k+2) on its own stream; [3..]: catch-up (host entry)
-    double* linv_all = nullptr; size_t linv_all_elems = 0;              // T' of every outer panel of the factorisation in flight (look-ahead): slot k = panel k
+    DevBuf<double> linv_all;                                            // T' of every outer panel of the factorisation in flight (look-ahead): slot k = panel k
     double* tslot(int k) const { return linv_all + (size_t)k * 128 * 128; }
-    cudaStream_t hp_stream = nullptr;                                   // stream of the panel chain (high priority)
-    cudaStream_t comm_stream = nullptr;                                 // collectives of the look-ahead schedule (high priority)
-    cudaStream_t aux_stream = nullptr;                                  // small side kernels of the wide chain (Rt = R2 R1, k_trecon), high priority
-    cudaEvent_t ev_aux[4] = {nullptr, nullptr, nullptr, nullptr};
-    cudaStream_t hp2_stream = nullptr;                                  // the chain's second apply (V_k -> columns of panel k+2), high priority
+    Stream hp_stream;                                                   // stream of the panel chain (high priority)
+    Stream comm_stream;                                                 // collectives of the look-ahead schedule (high priority)
+    Stream aux_stream;                                                  // small side kernels of the wide chain (Rt = R2 R1, k_trecon), high priority
+    Event ev_aux[4];
+    Stream hp2_stream;                                                  // the chain's second apply (V_k -> columns of panel k+2), high priority
     int host_trace = 0;                                                 // option: print a stage timeline of dhqr_qr_host_f64 to stderr
     int lookahead = 1;
-    unsigned long long* cells = nullptr;                                // panel exchange cells [IB+1][MAXG+1][IB][2]
+    DevBuf<unsigned long long> cells;                                   // panel exchange cells [IB+1][MAXG+1][IB][2]
     uint32_t ll_epoch = 0;
-    unsigned long long* cells2 = nullptr;                               // exchange cells of the panel kernel's fast path
-    int* fast_stats = nullptr;                                          // [2] fast / fallback panel counters
+    DevBuf<unsigned long long> cells2;                                  // exchange cells of the panel kernel's fast path
+    DevBuf<int> fast_stats;                                             // [2] fast / fallback panel counters
     int panel_fast = 1;
     int bs_wave_max_ctas = 0;                                           // co-residency limit of k_backsolve_wave on this device
-    unsigned long long* bs_cells = nullptr; size_t bs_cells_blocks = 0; // x cells of the wavefront ([block][32][2 words])
+    DevBuf<unsigned long long> bs_cells;                                // x cells of the wavefront ([block][32][2 words])
     uint32_t bs_epoch = 0;
-    unsigned int* uw_flags = nullptr; size_t uw_flags_n = 0; unsigned int uw_epoch = 0;   // k_unblocked_wave column flags
+    DevBuf<unsigned int> uw_flags; unsigned int uw_epoch = 0;           // k_unblocked_wave column flags
     // 128-column panel chain (dhqr_wide.cuh)
     int wide_panel = 1;                                                 // option: factor full aligned outer panels with CholeskyQR2 + reconstruction
-    WideCtl* wctl = nullptr;                                            // device control words (first refused panel, guards of the panel in flight)
-    double* wbuf = nullptr;                                             // R1, R2, X2, Rt, Y3 (plain 128x128) + XL, XL3 (rmul operand layout)
+    DevBuf<WideCtl> wctl;                                               // device control words (first refused panel, guards of the panel in flight)
+    DevBuf<double> wbuf;                                                // R1, R2, X2, Rt, Y3 (plain 128x128) + XL, XL3 (rmul operand layout)
     int64_t wide_panels = 0, wide_redone = 0;                           // statistics: panels factored by the wide chain / factorisations restarted
     double wide_kappa = 1000.0;                                         // guard on ||D R1^{-1}||_F of the first Cholesky factor (option "wide_kappa")
     // Q'b / Qb with one right-hand side: T' of every local panel (computed before the sweep), per-CTA partials of V'b, y, ticket
-    double* qt_T = nullptr;  size_t qt_T_elems = 0;
-    double* qt_part = nullptr; unsigned int* qt_ticket = nullptr;
+    DevBuf<double> qt_T;
+    DevBuf<double> qt_part; DevBuf<unsigned int> qt_ticket;
     int qt_vec = 1;                                                     // option: use it (0: the GEMM-shaped block update also for one right-hand side)
-    double* v1 = nullptr;    size_t v1_elems = 0;                       // unblocked path: v
-    double* xbuf = nullptr;  size_t xbuf_elems = 0;                     // back-substitution output
-    double* hostA = nullptr; size_t hostA_elems = 0;                    // device staging for _host_ entry points
-    double* hostB = nullptr; size_t hostB_elems = 0;
-    int64_t* d_i64 = nullptr;                                           // small int64 scratch (partition exchange)
+    DevBuf<double> v1;                                                  // unblocked path: v
+    DevBuf<double> xbuf;                                                // back-substitution output
+    DevBuf<double> hostA;                                               // device staging for _host_ entry points
+    DevBuf<double> hostB;
+    DevBuf<int64_t> d_i64;                                              // small int64 scratch (partition exchange)
     int64_t launches = 0;
-    cudaStream_t copy_stream = nullptr;      // compute stream of the _host_ entry points
-    cudaStream_t d2h_stream = nullptr;       // drains finished panels to the host while the factorisation continues
-    cudaStream_t h2d_stream = nullptr;       // uploads the later column chunks while the first ones are being factored
-    cudaStream_t cu_stream[CU_STREAMS] = {};   // catch-up: reflectors of finished panels applied to a column chunk that arrived late (chunks alternate)
+    Stream copy_stream;                      // compute stream of the _host_ entry points
+    Stream d2h_stream;                       // drains finished panels to the host while the factorisation continues
+    Stream h2d_stream;                       // uploads the later column chunks while the first ones are being factored
+    Stream cu_stream[CU_STREAMS];            // catch-up: reflectors of finished panels applied to a column chunk that arrived late (chunks alternate)
     // dhqr_qr_host_f64 -> look-ahead driver: column chunks still on their way to the device.  Chunk j = global columns [c0, c1),
     // usable once `ev` has fired, joins the trailing matrix at step `join` (after a catch-up with the reflectors of panels < join)
     struct UpChunk { int64_t c0, c1; cudaEvent_t ev; int join; };
@@ -164,7 +218,7 @@ struct dhqr_context {
     int host_first = 0;                      // option: columns of the first upload (0: three panels)
     int host_h2d_gbs = 50, host_tflops = 27; // option: what the join-step planner assumes about the link and the device
     int host_chain_us = 300;                 // option: ... and about the duration of a step of the schedule while the window is narrow
-    std::vector<cudaEvent_t> panel_events;
+    std::vector<Event> panel_events;
     // set by dhqr_qr_host_f64: finished columns are copied back as soon as their panel is final
     double* mirror_host = nullptr;
     int64_t mirror_lda = 0;
@@ -172,11 +226,11 @@ struct dhqr_context {
     bool attrs_set = false;
     // per-kernel-class CUDA-event profiling (option "profile")
     int profile = 0;
-    struct ProfRec { int slot; cudaEvent_t e0, e1; };
+    struct ProfRec { int slot; Event e0, e1; };
     struct ProfSlot { const char* name; double ms = 0.0; int64_t count = 0; double work = 0.0; };
     std::vector<ProfRec> prof_pending;
     std::vector<ProfSlot> prof_slots;
-    cudaEvent_t prof_open = nullptr;
+    Event prof_open;
 };
 
 static constexpr int NBMAX = 128;
@@ -221,18 +275,6 @@ static int set_attrs(dhqr_context* c) {
     return 0;
 }
 
-template <typename T>
-static int ensure(T** p, size_t* have, size_t need) {
-    if (*have >= need && *p) return 0;
-    if (*p) CU(cudaFree(*p));
-    *p = nullptr;
-    *have = 0;
-    CU(cudaMalloc((void**)p, need * sizeof(T)));
-    CU(cudaMemset(*p, 0, need * sizeof(T)));
-    *have = need;
-    return 0;
-}
-
 static constexpr int64_t WPART_TILES = 2304;   // capacity of the partial buffer in 128 x 64 tiles (151 MB per set)
 
 // npanels: outer panels of the factorisation about to run (T' slots of the look-ahead schedule); catchup: also size the fourth
@@ -240,40 +282,31 @@ static constexpr int64_t WPART_TILES = 2304;   // capacity of the partial buffer
 static int ensure_workspace(dhqr_context* c, int64_t m, int64_t n_local_max, int64_t npanels = 0, bool catchup = false) {
     TRY(set_attrs(c));
     const int64_t vrows = rup(m, 128) + 128;
-    if (c->vrows_cap < vrows || !c->vpk2[0]) {
-        for (int b = 0; b < 3; ++b) TRY(ensure(&c->vpk2[b], &c->vpk_elems[b], (size_t)(vrows / KC1) * VPK_CHUNK));
-        c->vrows_cap = vrows;
-    }
-    if (catchup) for (int b = 3; b < 3 + CU_STREAMS; ++b) TRY(ensure(&c->vpk2[b], &c->vpk_elems[b], (size_t)(vrows / KC1) * VPK_CHUNK));
-    TRY(ensure(&c->linv_all, &c->linv_all_elems, (size_t)std::max<int64_t>(npanels, 4) * NBMAX * NBMAX));
+    for (int b = 0; b < (catchup ? 3 + CU_STREAMS : 3); ++b) TRY(c->vpk2[b].grow((size_t)(vrows / KC1) * VPK_CHUNK));
+    TRY(c->linv_all.grow((size_t)std::max<int64_t>(npanels, 4) * NBMAX * NBMAX));
     const int64_t tiles_max = (n_local_max + NBMAX + G1_BN - 1) / G1_BN + 1;
     for (int b = 0; b < (catchup ? 3 + CU_STREAMS : 3); ++b) {
         auto& w = c->ws[b];
         // set 2 only ever updates the <= 128 columns of one panel: a quarter of the split-K partial buffer is plenty
-        TRY(ensure(&w.wpart, &w.wpart_elems, (size_t)(b != 2 ? std::max(WPART_TILES, tiles_max) : WPART_TILES / 4) * NBMAX * G1_BN));
-        TRY(ensure(&w.wsum, &w.wsum_elems, (size_t)NBMAX * (rup(n_local_max + NBMAX, 128) + 128)));
-        TRY(ensure(&w.ypk, &w.ypk_elems, (size_t)(NBMAX / KC) * YT * LDK * ((n_local_max + YT - 1) / YT + 2)));
-        TRY(ensure(&w.linv, &w.linv_elems, (size_t)NBMAX * NBMAX));
+        TRY(w.wpart.grow((size_t)(b != 2 ? std::max(WPART_TILES, tiles_max) : WPART_TILES / 4) * NBMAX * G1_BN));
+        TRY(w.wsum.grow((size_t)NBMAX * (rup(n_local_max + NBMAX, 128) + 128)));
+        TRY(w.ypk.grow((size_t)(NBMAX / KC) * YT * LDK * ((n_local_max + YT - 1) / YT + 2)));
+        TRY(w.linv.grow((size_t)NBMAX * NBMAX));
     }
-    size_t one = 0;
-    if (!c->cells2) {
-        const size_t words = (2 * (size_t)(PANEL_MAXG + 1) * (IB * (IB + 1) / 2) + IB * IB + 2 * IB) * 2;
-        CU(cudaMalloc((void**)&c->cells2, words * sizeof(unsigned long long)));
-        CU(cudaMemset(c->cells2, 0, words * sizeof(unsigned long long)));
-        CU(cudaMalloc((void**)&c->fast_stats, 2 * sizeof(int)));
-        CU(cudaMemset(c->fast_stats, 0, 2 * sizeof(int)));
-        c->ll_epoch = 0;
-    }
-    if (!c->cells) { one = 0; TRY(ensure(&c->cells, &one, (size_t)IB * (PANEL_MAXG + 2) * IB * 2)); c->ll_epoch = 0; }
-    if (!c->wctl) {
-        CU(cudaMalloc((void**)&c->wctl, sizeof(WideCtl)));
+    bool fresh2 = false, fresh = false;   // new exchange cells: the tags start over
+    TRY(c->cells2.grow((2 * (size_t)(PANEL_MAXG + 1) * (IB * (IB + 1) / 2) + IB * IB + 2 * IB) * 2, &fresh2));
+    TRY(c->fast_stats.grow(2));
+    TRY(c->cells.grow((size_t)IB * (PANEL_MAXG + 2) * IB * 2, &fresh));
+    if (fresh2 || fresh) c->ll_epoch = 0;
+    bool fresh_ctl = false;
+    TRY(c->wctl.grow(1, &fresh_ctl));
+    if (fresh_ctl) {
         const WideCtl init = {W_NOFAIL, 0, {0, 0}};
         CU(cudaMemcpy(c->wctl, &init, sizeof(init), cudaMemcpyHostToDevice));
-        size_t o3 = 0;
-        TRY(ensure(&c->wbuf, &o3, (size_t)5 * WP * WP + 3 * XL_ELEMS));
     }
-    TRY(ensure(&c->v1, &c->v1_elems, (size_t)2 * rup(m + 4, 2)));
-    TRY(ensure(&c->xbuf, &c->xbuf_elems, (size_t)1));
+    TRY(c->wbuf.grow((size_t)5 * WP * WP + 3 * XL_ELEMS));
+    TRY(c->v1.grow((size_t)2 * rup(m + 4, 2)));
+    TRY(c->xbuf.grow(1));
     return 0;
 }
 
@@ -288,7 +321,7 @@ static int prof_slot(dhqr_context* c, const char* name) {
 // pre(): open a CUDA-event bracket on the launching stream when profiling is on
 static void pre(dhqr_context* c, cudaStream_t st) {
     if (!c->profile) return;
-    cudaEventCreate(&c->prof_open);
+    c->prof_open.create(cudaEventDefault);
     cudaEventRecord(c->prof_open, st);
 }
 static int post(dhqr_context* c, cudaStream_t st, const char* what, double work = 0.0) {
@@ -296,12 +329,11 @@ static int post(dhqr_context* c, cudaStream_t st, const char* what, double work 
     if (c->profile && c->prof_open) {
         dhqr_context::ProfRec r;
         r.slot = prof_slot(c, what);
-        r.e0 = c->prof_open;
-        cudaEventCreate(&r.e1);
+        r.e0 = std::move(c->prof_open);
+        r.e1.create(cudaEventDefault);
         cudaEventRecord(r.e1, st);
-        c->prof_pending.push_back(r);
         c->prof_slots[r.slot].work += work;
-        c->prof_open = nullptr;
+        c->prof_pending.push_back(std::move(r));
     }
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return set_err(1000 + (int)e, "launch of %s failed: %s", what, cudaGetErrorString(e));
@@ -348,10 +380,10 @@ static int apply_block_reflector(dhqr_context* c, cudaStream_t st, const double*
     const int next = nv + ncols;
     const int tiles = (next + bn - 1) / bn;
     const int nchunks = (int)((rows + KC1 - 1) / KC1);
-    const int nsplit = pick_splits(tiles, nchunks, c->sms, (int64_t)(w.wpart_elems / ((size_t)bn * NBPK)));
+    const int nsplit = pick_splits(tiles, nchunks, c->sms, (int64_t)(w.wpart.size() / ((size_t)bn * NBPK)));
     const int64_t pstride = (int64_t)tiles * bn * NBPK;
-    if ((size_t)(pstride * nsplit) > w.wpart_elems) return set_err(4001, "internal: W partial workspace too small");
-    if ((size_t)next * NBPK > w.wsum_elems) return set_err(4003, "internal: W workspace too small");
+    if ((size_t)(pstride * nsplit) > w.wpart.size()) return set_err(4001, "internal: W partial workspace too small");
+    if ((size_t)next * NBPK > w.wsum.size()) return set_err(4003, "internal: W workspace too small");
     GemmVtaArgs g1;
     g1.vpk = vpk; g1.voff = voff; g1.nv = nv;
     g1.A = C; g1.lda = ldc; g1.rows = rows; g1.na = ncols; g1.nchunks = nchunks;
@@ -420,8 +452,8 @@ static int launch_panel(dhqr_context* c, cudaStream_t st, double* vpk, double* P
     const size_t smem = (size_t)IB * lds * 8;
     if (smem > 184 * 1024) return set_err(-2, "m too large for the resident panel kernel (%lld rows per CTA)", (long long)rpc);
     if (c->ll_epoch > 0xF0000000u) {   // tag space nearly used up: start over with clean cells
-        CU(cudaMemsetAsync(c->cells, 0, sizeof(unsigned long long) * (size_t)IB * (PANEL_MAXG + 2) * IB * 2, st));
-        CU(cudaMemsetAsync(c->cells2, 0, sizeof(unsigned long long) * (2 * (size_t)(PANEL_MAXG + 1) * (IB * (IB + 1) / 2) + IB * IB + 2 * IB) * 2, st));
+        CU(cudaMemsetAsync(c->cells, 0, sizeof(unsigned long long) * c->cells.size(), st));
+        CU(cudaMemsetAsync(c->cells2, 0, sizeof(unsigned long long) * c->cells2.size(), st));
         c->ll_epoch = 0;
     }
     PanelArgs a;
@@ -487,6 +519,14 @@ static int check_common(dhqr_context* c, int64_t m, int64_t n_global, int64_t co
     return 0;
 }
 
+// right-hand sides b (m x nrhs): a bad argument is refused with minus its position in the entry point's argument list
+static int check_rhs(int64_t m, int nrhs, const void* b, int64_t ldb, int idx_b, int idx_ldb, int idx_nrhs) {
+    if (nrhs < 0) return set_err(-idx_nrhs, "nrhs < 0");
+    if (nrhs > 0 && !b) return set_err(-idx_b, "null b");
+    if (ldb < std::max<int64_t>(1, m)) return set_err(-idx_ldb, "ldb < max(1,m)");
+    return 0;
+}
+
 // ------------------------------------------------------------------------------------------------
 // qr!: blocked driver  (S:113-148, S:198-213)
 // ------------------------------------------------------------------------------------------------
@@ -498,6 +538,17 @@ static PanelGeom panel_geom(const Panel& p, int64_t m) {
     g.vrows = rup(g.rows, 128);
     g.nbp = (int)rup(p.kb, IB);
     return g;
+}
+
+// Packs the kb columns of the panel at src (mp rows; tril: zeros above the diagonal, where a factored panel keeps R) into vpk
+// with panel row 0 at window row vtop.  packed_cols (32 or 128) columns are written, those beyond kb as zeros: they must
+// cover the nbp the block update then reads.
+static int pack_panel(dhqr_context* c, cudaStream_t st, const double* src, int64_t lda, int64_t mp, int kb, int tril, double* vpk,
+                      int64_t vtop, int64_t vrows, int packed_cols) {
+    dim3 grid((unsigned)std::min<int64_t>((vrows / 4 + 255) / 256, 4 * c->sms), packed_cols);
+    pre(c, st);
+    k_pack<<<grid, 256, 0, st>>>(src, lda, mp, kb, tril, vpk, 0, vtop, vrows);
+    return post(c, st, "k_pack");
 }
 
 // factor one outer panel on stream st: inner panels of IB columns + updates inside the outer panel; V -> vpk
@@ -530,7 +581,7 @@ static int launch_panel_gram(dhqr_context* c, cudaStream_t st, const double* vpk
     pre(c, st);
     const int cps = std::max(1, (nchunks + c->sms - 1) / c->sms);                           // chunks per CTA: whole waves of equal CTAs
     const int nsplit = (nchunks + cps - 1) / cps;
-    if ((size_t)nsplit * pstride > w.wpart_elems) return set_err(4001, "internal: W partial workspace too small");
+    if ((size_t)nsplit * pstride > w.wpart.size()) return set_err(4001, "internal: W partial workspace too small");
     GramSymArgs g;
     g.vpk = vpk; g.nchunks = nchunks; g.Wp = w.wpart; g.pstride = pstride;
     k_gram_sym<<<nsplit, (GS_MMA_WARPS + 1) * 32, SMEM_GRAM_SYM, st>>>(g);
@@ -564,10 +615,7 @@ static int factor_outer_panel_wide(dhqr_context* c, cudaStream_t st, double* vpk
     int nsplit = 0;
     int64_t pstride = 0;
     auto gram = [&]() -> int { return launch_panel_gram(c, st, vpk, w, g.rows, &nsplit, &pstride); };
-    pre(c, st);
-    dim3 pgrid((unsigned)std::min<int64_t>((g.vrows / 4 + 255) / 256, 4 * c->sms), WP);
-    k_pack<<<pgrid, 256, 0, st>>>(P, lda, g.rows, WP, 0, vpk, 0, 0, g.vrows);
-    TRY(post(c, st, "k_pack"));
+    TRY(pack_panel(c, st, P, lda, g.rows, WP, 0, vpk, 0, g.vrows, WP));
     TRY(gram());
     pre(c, st);
     k_wreduce4<<<(WP * WP * 4) / 256, 256, 0, st>>>(w.wpart, pstride, nsplit, (int64_t)WP * WP, w.wsum);
@@ -622,9 +670,8 @@ static int factor_outer_panel(dhqr_context* c, cudaStream_t st, double* vpk, dhq
 static int mirror_panel_to_host(dhqr_context* c, cudaStream_t st, const Panel& p, int64_t m, int64_t col0, const double* A,
                                 int64_t lda) {
     if (!c->mirror_host) return 0;   // host entry point only: this panel's columns are final -> start their D2H now
-    cudaEvent_t ev;
-    CU(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-    c->panel_events.push_back(ev);
+    Event& ev = c->panel_events.emplace_back();
+    CU(ev.create(cudaEventDisableTiming));
     CU(cudaEventRecord(ev, st));
     CU(cudaStreamWaitEvent(c->d2h_stream, ev, 0));
     CU(cudaMemcpy2DAsync(c->mirror_host + p.c * c->mirror_lda, (size_t)c->mirror_lda * 8, A + (p.c - col0) * lda, (size_t)lda * 8,
@@ -685,16 +732,17 @@ static int qr_blocked_lookahead(dhqr_context* c, cudaStream_t st, int64_t m, int
     const int64_t lend = col0 + nl;
     const int K = (int)panels.size(), K0 = pl.kstart;
     cudaStream_t hp = c->hp_stream;
-    std::vector<cudaEvent_t> evPanel(K), evNext(K), evBulk(K), evA2(K);
+    // the events of this call: destroyed on return, when the work they order is enqueued
+    std::vector<Event> evPanel(K), evNext(K), evBulk(K), evA2(K), evHp(K), evCatch;
     std::vector<char> haveA2(K, 0);
     // stage timeline of the pipelined host entry (option host_trace; dhqr_qr_host_f64 is the only caller that mirrors to the host)
     const bool trace = c->host_trace && c->mirror_host;
     const unsigned evflags = trace ? cudaEventDefault : cudaEventDisableTiming;
     for (int k = K0; k < K; ++k) {
-        CU(cudaEventCreateWithFlags(&evA2[k], cudaEventDisableTiming));
-        CU(cudaEventCreateWithFlags(&evPanel[k], evflags));
-        CU(cudaEventCreateWithFlags(&evNext[k], evflags));
-        CU(cudaEventCreateWithFlags(&evBulk[k], evflags));
+        CU(evA2[k].create(cudaEventDisableTiming));
+        CU(evPanel[k].create(evflags));
+        CU(evNext[k].create(evflags));
+        CU(evBulk[k].create(evflags));
     }
     // local intersection of the global column range [a, b) -> pointer + count
     auto clip = [&](int64_t a, int64_t b, int64_t& lo, int64_t& hi) { lo = std::max(a, col0); hi = std::min(b, lend); return hi > lo; };
@@ -703,12 +751,11 @@ static int qr_blocked_lookahead(dhqr_context* c, cudaStream_t st, int64_t m, int
     // evPanel[k].  The comm stream first waits for everything queued on hp so far: on the owner that is the factorisation of
     // panel k, on every rank the last reads of the ring slot's previous occupant V_{k-3}.
     cudaStream_t cs = c->comm_stream;
-    std::vector<cudaEvent_t> evHp(K, nullptr);
     auto publish = [&](int k) -> int {
         if (c->nranks > 1) {
             const PanelGeom g = panel_geom(panels[k], m);
             double* v = c->vpk2[k % 3];
-            CU(cudaEventCreateWithFlags(&evHp[k], cudaEventDisableTiming));
+            CU(evHp[k].create(cudaEventDisableTiming));
             CU(cudaEventRecord(evHp[k], hp));
             CU(cudaStreamWaitEvent(cs, evHp[k], 0));
             NC(g_nccl.Broadcast(v, v, (size_t)(g.vrows / KC1) * VPK_CHUNK, ncclFloat64, panels[k].owner, c->comm, cs));
@@ -748,32 +795,29 @@ static int qr_blocked_lookahead(dhqr_context* c, cudaStream_t st, int64_t m, int
             const PanelGeom gq = panel_geom(pq, m);
             cudaStreamWaitEvent(cu, evPanel[q], 0);                   // V_q is final in A ...
             cudaStreamWaitEvent(cu, evNext[q], 0);                    // ... and T'_q sits in its slot
-            dim3 grid((unsigned)std::min<int64_t>((gq.vrows / 4 + 255) / 256, 4 * c->sms), gq.nbp <= IB ? IB : NBMAX);
-            k_pack<<<grid, 256, 0, cu>>>(A + (pq.c - col0) * lda + pq.c, lda, m - pq.c, pq.kb, 1, vpk_cu, 0, pq.c - gq.r0, gq.vrows);
-            TRY(post(c, cu, "k_pack"));
+            TRY(pack_panel(c, cu, A + (pq.c - col0) * lda + pq.c, lda, m - pq.c, pq.kb, 1, vpk_cu, pq.c - gq.r0, gq.vrows,
+                           gq.nbp <= IB ? IB : NBMAX));
             TRY(apply_block_reflector(c, cu, vpk_cu, ws_cu, 0, gq.nbp, gq.rows, pq.c - gq.r0, A + (u.c0 - col0) * lda + gq.r0, lda,
                                       (int)(u.c1 - u.c0), haveTslot[q] != 0, c->tslot(q), q + 1));
         }
         cudaEventRecord(done, cu);
         return 0;
     };
-    std::vector<cudaEvent_t> evCatch;
     std::vector<int> joinedAt;
-    int rc = 0;
-    cudaEvent_t fork = nullptr, hpdone = nullptr;
-    do {
-        if (cudaEventCreateWithFlags(&fork, evflags) != cudaSuccess) { rc = set_err(1001, "event create failed"); break; }
+    const int rc = [&]() -> int {
+        Event fork;
+        CU(fork.create(evflags));
         cudaEventRecord(fork, st);
         cudaStreamWaitEvent(hp, fork, 0);                          // hp starts after everything already queued on st
         std::vector<char> ownT(K, 0);       // T'_k already sits in the ring slot on this rank (wide panel factored here, k_trecon)
         if (c->rank == panels[K0].owner) {
             const bool wide = plan_wide(c, pl, panels, K0, m);
-            if ((rc = factor_outer_panel(c, hp, c->vpk2[K0 % 3], c->ws[1], panels[K0], m, col0, A, lda, alpha, K0, wide, c->tslot(K0)))) break;
-            if ((rc = mirror_panel_to_host(c, hp, panels[K0], m, col0, A, lda))) break;
+            TRY(factor_outer_panel(c, hp, c->vpk2[K0 % 3], c->ws[1], panels[K0], m, col0, A, lda, alpha, K0, wide, c->tslot(K0)));
+            TRY(mirror_panel_to_host(c, hp, panels[K0], m, col0, A, lda));
             if (wide) { ownT[K0] = 1; cudaEventRecord(evNext[K0], hp); }
         }
-        if ((rc = publish(K0))) break;
-        for (int k = K0; k < K && !rc; ++k) {
+        TRY(publish(K0));
+        for (int k = K0; k < K; ++k) {
             const Panel& p = panels[k];
             const PanelGeom g = panel_geom(p, m);
             const double* vk = c->vpk2[k % 3];
@@ -788,17 +832,15 @@ static int qr_blocked_lookahead(dhqr_context* c, cudaStream_t st, int64_t m, int
                 const int64_t t3 = k + 3 < K ? panels[k + 3].c + panels[k + 3].kb : lend;   // end of panel k+3
                 while (upnext < c->up_chunks.size() && (c->up_chunks[upnext].join <= k || c->up_chunks[upnext].c0 < t3)) {
                     const auto& u = c->up_chunks[upnext];
-                    if (u.c0 < t2 || u.c0 != wend) { rc = set_err(4005, "internal: upload chunk %d joins too late (step %d)", (int)upnext, k); break; }
-                    cudaEvent_t done;
-                    if (cudaEventCreateWithFlags(&done, evflags) != cudaSuccess) { rc = set_err(1001, "event create failed"); break; }
-                    evCatch.push_back(done);
+                    if (u.c0 < t2 || u.c0 != wend) return set_err(4005, "internal: upload chunk %d joins too late (step %d)", (int)upnext, k);
+                    Event& done = evCatch.emplace_back();
+                    CU(done.create(evflags));
                     joinedAt.push_back(k);
-                    if ((rc = catch_up(u, (int)(upnext % CU_STREAMS), k, done))) break;
+                    TRY(catch_up(u, (int)(upnext % CU_STREAMS), k, done));
                     wend = u.c1;
                     ++upnext;
                 }
-                if (rc) break;
-                if (wend < t2) { rc = set_err(4005, "internal: window ends at %lld before panel %d", (long long)wend, k + 2); break; }
+                if (wend < t2) return set_err(4005, "internal: window ends at %lld before panel %d", (long long)wend, k + 2);
             }
             double* lk = c->tslot(k);
             bool haveT = ownT[k];                                        // T'_k in lk (this rank)
@@ -814,18 +856,18 @@ static int qr_blocked_lookahead(dhqr_context* c, cudaStream_t st, int64_t m, int
                     if (k - 1 >= K0 && haveA2[k - 1]) cudaStreamWaitEvent(hp, evA2[k - 1], 0);   // V_{k-1} reached these columns
                     if (clip(t0, t1, lo, hi)) {
                         const bool hadT = haveT;
-                        if ((rc = apply_block_reflector(c, hp, vk, c->ws[1], 0, g.nbp, g.rows, p.c - g.r0, A + (lo - col0) * lda + g.r0,
-                                                        lda, (int)(hi - lo), haveT, lk, k + 1))) break;
+                        TRY(apply_block_reflector(c, hp, vk, c->ws[1], 0, g.nbp, g.rows, p.c - g.r0, A + (lo - col0) * lda + g.r0, lda,
+                                                  (int)(hi - lo), haveT, lk, k + 1));
                         haveT = true;
                         if (!hadT) cudaEventRecord(evNext[k], hp);       // T'_k is in the ring: the bulk update may start
                     }
                     const bool widen = plan_wide(c, pl, panels, k + 1, m);
-                    if ((rc = factor_outer_panel(c, hp, c->vpk2[(k + 1) % 3], c->ws[1], panels[k + 1], m, col0, A, lda, alpha, k + 1, widen,
-                                                 c->tslot(k + 1)))) break;
+                    TRY(factor_outer_panel(c, hp, c->vpk2[(k + 1) % 3], c->ws[1], panels[k + 1], m, col0, A, lda, alpha, k + 1, widen,
+                                           c->tslot(k + 1)));
                     if (widen) { ownT[k + 1] = 1; cudaEventRecord(evNext[k + 1], hp); }
-                    if ((rc = mirror_panel_to_host(c, hp, panels[k + 1], m, col0, A, lda))) break;
+                    TRY(mirror_panel_to_host(c, hp, panels[k + 1], m, col0, A, lda));
                 }
-                if ((rc = publish(k + 1))) break;
+                TRY(publish(k + 1));
             }
             // columns of panel k+2: their V_0..V_{k-1} come from the bulk updates up to k-1.  This apply is off the chain's
             // stream (it overlaps the factorisation of panel k+1); the chain picks it up through evA2[k] before it applies
@@ -837,8 +879,8 @@ static int qr_blocked_lookahead(dhqr_context* c, cudaStream_t st, int64_t m, int
                 if (k - 1 >= K0) cudaStreamWaitEvent(s2, evBulk[k - 1], 0);
                 wait_panel(s2, k);
                 const bool hadT = haveT;
-                if ((rc = apply_block_reflector(c, s2, vk, c->ws[2], 0, g.nbp, g.rows, p.c - g.r0, A + (lo - col0) * lda + g.r0, lda,
-                                                (int)(hi - lo), haveT, lk, k + 1))) break;
+                TRY(apply_block_reflector(c, s2, vk, c->ws[2], 0, g.nbp, g.rows, p.c - g.r0, A + (lo - col0) * lda + g.r0, lda,
+                                          (int)(hi - lo), haveT, lk, k + 1));
                 haveT = true;
                 if (!hadT) cudaEventRecord(evNext[k], s2);               // T'_k came from this apply
                 cudaEventRecord(evA2[k], s2);
@@ -848,21 +890,19 @@ static int qr_blocked_lookahead(dhqr_context* c, cudaStream_t st, int64_t m, int
             wait_panel(st, k);
             if (clip(t2, std::min(lend, wold), lo, hi)) {
                 if (haveT) cudaStreamWaitEvent(st, evNext[k], 0);
-                if ((rc = apply_block_reflector(c, st, vk, c->ws[0], 0, g.nbp, g.rows, p.c - g.r0, A + (lo - col0) * lda + g.r0, lda,
-                                                (int)(hi - lo), haveT, haveT ? lk : nullptr, k + 1))) break;
+                TRY(apply_block_reflector(c, st, vk, c->ws[0], 0, g.nbp, g.rows, p.c - g.r0, A + (lo - col0) * lda + g.r0, lda,
+                                          (int)(hi - lo), haveT, haveT ? lk : nullptr, k + 1));
             }
-            for (size_t j = up0; j < upnext && !rc; ++j) {             // the chunks that joined at this step, each behind its catch-up
+            for (size_t j = up0; j < upnext; ++j) {                      // the chunks that joined at this step, each behind its catch-up
                 const auto& u = c->up_chunks[j];
                 cudaStreamWaitEvent(st, evCatch[j], 0);
                 if (haveT) cudaStreamWaitEvent(st, evNext[k], 0);
-                rc = apply_block_reflector(c, st, vk, c->ws[0], 0, g.nbp, g.rows, p.c - g.r0, A + (u.c0 - col0) * lda + g.r0, lda,
-                                           (int)(u.c1 - u.c0), haveT, haveT ? lk : nullptr, k + 1);
+                TRY(apply_block_reflector(c, st, vk, c->ws[0], 0, g.nbp, g.rows, p.c - g.r0, A + (u.c0 - col0) * lda + g.r0, lda,
+                                          (int)(u.c1 - u.c0), haveT, haveT ? lk : nullptr, k + 1));
             }
-            if (rc) break;
             haveTslot[k] = haveT;
             cudaEventRecord(evBulk[k], st);
         }
-        if (rc) break;
         cudaStreamWaitEvent(st, evPanel[K - 1], 0);                // join: alpha and the last panel come from hp / the comm stream
         if (c->nranks > 1) {
             cudaEventRecord(evHp[K - 1], hp);                      // (re-recorded: everything queued on hp)
@@ -887,9 +927,11 @@ static int qr_blocked_lookahead(dhqr_context* c, cudaStream_t st, int64_t m, int
                 fprintf(stderr, "[dhqr host] step %2d: panel %7.2f  T' %7.2f  bulk %7.2f ms\n", k, tp, tt, tb);
             }
         }
-    } while (0);
+        return 0;
+    }();
     // error path: the caller's stream must not run ahead of (or return before) work already queued on the internal stream
-    if (rc && cudaEventCreateWithFlags(&hpdone, cudaEventDisableTiming) == cudaSuccess) {
+    Event hpdone;
+    if (rc && hpdone.create(cudaEventDisableTiming) == cudaSuccess) {
         cudaEventRecord(hpdone, hp);
         cudaStreamWaitEvent(st, hpdone, 0);
         cudaEventRecord(hpdone, cs);
@@ -900,19 +942,11 @@ static int qr_blocked_lookahead(dhqr_context* c, cudaStream_t st, int64_t m, int
             cudaEventRecord(hpdone, c->cu_stream[i]);
             cudaStreamWaitEvent(st, hpdone, 0);
         }
-        cudaEventDestroy(hpdone);
     }
-    for (cudaEvent_t e : evHp)
-        if (e) cudaEventDestroy(e);
-    for (cudaEvent_t e : evCatch) cudaEventDestroy(e);
-    // events may be destroyed once recorded/waited on: the work they order is already enqueued
-    if (fork) cudaEventDestroy(fork);
-    for (int k = K0; k < K; ++k) { cudaEventDestroy(evPanel[k]); cudaEventDestroy(evNext[k]); cudaEventDestroy(evBulk[k]); cudaEventDestroy(evA2[k]); }
-    if (!rc) {
-        cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) rc = set_err(1000 + (int)e, "look-ahead enqueue failed: %s", cudaGetErrorString(e));
-    }
-    return rc;
+    if (rc) return rc;
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return set_err(1000 + (int)e, "look-ahead enqueue failed: %s", cudaGetErrorString(e));
+    return 0;
 }
 
 // largest row count the resident 32-column panel kernel can take on this device (slab of rows in shared memory)
@@ -959,7 +993,7 @@ static int qr_blocked(dhqr_context* c, cudaStream_t st, int64_t m, int64_t n, in
         // learn whether a panel was refused; if so, everything from that panel on was skipped on the device and is redone
         // here, that panel with the 32-column chain (same result on every rank: the verdict travels with the V buffer).
         int fail = W_NOFAIL;
-        CU(cudaMemcpyAsync(&fail, &c->wctl->fail_step, sizeof(int), cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(&fail, &((WideCtl*)c->wctl)->fail_step, sizeof(int), cudaMemcpyDeviceToHost, st));
         CU(cudaStreamSynchronize(st));
         if (fail == W_NOFAIL) return 0;
         if (fail < pl.kstart || fail >= (int)panels.size()) return set_err(4004, "internal: bad restart index %d", fail);
@@ -979,18 +1013,14 @@ static int qr_unblocked(dhqr_context* c, cudaStream_t st, int64_t m, int64_t n, 
     const int64_t lend = col0 + nl;
     if (c->nranks == 1 && n > 0 && m <= (int64_t)UW_MAXI * UW_THREADS && !c->profile && !c->sync) {
         // single GPU, short columns: the whole column loop as one persistent cooperative launch (k_unblocked_wave)
-        if (c->uw_flags_n < (size_t)n) {
-            if (c->uw_flags) CU(cudaFree(c->uw_flags));
-            c->uw_flags = nullptr;
-            CU(cudaMalloc((void**)&c->uw_flags, sizeof(unsigned int) * (size_t)(n + 64)));
-            CU(cudaMemset(c->uw_flags, 0, sizeof(unsigned int) * (size_t)(n + 64)));
-            c->uw_flags_n = (size_t)n + 64;
-            c->uw_epoch = 0;
-        }
-        if (c->uw_epoch > 0xFFFFFFF0u) { CU(cudaMemsetAsync(c->uw_flags, 0, sizeof(unsigned int) * c->uw_flags_n, st)); c->uw_epoch = 0; }
+        bool fresh = false;   // new flags (64 spare): the tags start over
+        if (c->uw_flags.size() < (size_t)n) TRY(c->uw_flags.grow((size_t)n + 64, &fresh));
+        if (fresh) c->uw_epoch = 0;
+        if (c->uw_epoch > 0xFFFFFFF0u) { CU(cudaMemsetAsync(c->uw_flags, 0, sizeof(unsigned int) * c->uw_flags.size(), st)); c->uw_epoch = 0; }
         const unsigned int tag = ++c->uw_epoch;
         int nn = (int)n;
-        void* args[] = {&A, &lda, &m, &nn, &alpha, &c->uw_flags, (void*)&tag};
+        unsigned int* flags = c->uw_flags;
+        void* args[] = {&A, &lda, &m, &nn, &alpha, &flags, (void*)&tag};
         const int G = (int)std::min<int64_t>(c->sms, n);
         pre(c, st);
         cudaError_t e = cudaLaunchCooperativeKernel((void*)k_unblocked_wave, dim3(G), dim3(UW_THREADS), args, 0, st);
@@ -1074,13 +1104,10 @@ static int apply_qt_local(dhqr_context* c, cudaStream_t st, int64_t m, int64_t c
     for (int64_t o = ofirst; o >= 0 && o < nl; o += ostep) {
         const int kb = (int)std::min<int64_t>(NBMAX, nl - o);
         const int64_t cs = col0 + o;
-        const int64_t r0 = cs & ~(int64_t)31;
-        const int64_t rows = m - r0, vrows = rup(rows, 128);
+        const PanelGeom g = panel_geom({0, cs, kb}, m);
         const int nbp = kb <= IB ? IB : NBMAX;
-        dim3 grid((unsigned)std::min<int64_t>((vrows / 4 + 255) / 256, 4 * c->sms), nbp);
-        k_pack<<<grid, 256, 0, st>>>(A + o * lda + cs, lda, m - cs, kb, 1, c->vpk2[0], 0, cs - r0, vrows);
-        TRY(post(c, st, "k_pack"));
-        TRY(apply_block_reflector(c, st, c->vpk2[0], c->ws[0], 0, nbp, rows, cs - r0, b + r0, ldb, nrhs, false, nullptr, 0, notrans));
+        TRY(pack_panel(c, st, A + o * lda + cs, lda, m - cs, kb, 1, c->vpk2[0], cs - g.r0, g.vrows, nbp));
+        TRY(apply_block_reflector(c, st, c->vpk2[0], c->ws[0], 0, nbp, g.rows, cs - g.r0, b + g.r0, ldb, nrhs, false, nullptr, 0, notrans));
     }
     return 0;
 }
@@ -1091,25 +1118,19 @@ static constexpr int QT_MAXG = 1024;
 static int qt_prepare(dhqr_context* c, cudaStream_t st, int64_t m, int64_t col0, int64_t nl, const double* A, int64_t lda) {
     const int npl = (int)((nl + NBMAX - 1) / NBMAX);
     if (npl <= 0) return 0;
-    TRY(ensure(&c->qt_T, &c->qt_T_elems, (size_t)npl * NBMAX * NBMAX));
-    if (!c->qt_part) {
-        CU(cudaMalloc((void**)&c->qt_part, sizeof(double) * (size_t)(QT_MAXG + 1) * WP));     // last row: y
-        CU(cudaMalloc((void**)&c->qt_ticket, sizeof(unsigned int)));
-        CU(cudaMemset(c->qt_ticket, 0, sizeof(unsigned int)));
-    }
+    TRY(c->qt_T.grow((size_t)npl * NBMAX * NBMAX));
+    TRY(c->qt_part.grow((size_t)(QT_MAXG + 1) * WP));     // last row: y
+    TRY(c->qt_ticket.grow(1));
     auto& w = c->ws[0];
-    if ((size_t)npl * NBMAX * NBMAX > w.wsum_elems) return set_err(4006, "internal: Gram workspace too small");
+    if ((size_t)npl * NBMAX * NBMAX > w.wsum.size()) return set_err(4006, "internal: Gram workspace too small");
     for (int p = 0; p < npl; ++p) {
-        const int64_t o = (int64_t)p * NBMAX, cs = col0 + o, r0 = cs & ~(int64_t)31;
+        const int64_t o = (int64_t)p * NBMAX, cs = col0 + o;
         const int kb = (int)std::min<int64_t>(NBMAX, nl - o);
-        const int64_t rows = m - r0, vrows = rup(rows, 128);
-        dim3 grid((unsigned)std::min<int64_t>((vrows / 4 + 255) / 256, 4 * c->sms), NBMAX);
-        pre(c, st);
-        k_pack<<<grid, 256, 0, st>>>(A + o * lda + cs, lda, m - cs, kb, 1, c->vpk2[0], 0, cs - r0, vrows);
-        TRY(post(c, st, "k_pack"));
+        const PanelGeom g = panel_geom({0, cs, kb}, m);
+        TRY(pack_panel(c, st, A + o * lda + cs, lda, m - cs, kb, 1, c->vpk2[0], cs - g.r0, g.vrows, NBMAX));
         int nsplit = 0;
         int64_t pstride = 0;
-        TRY(launch_panel_gram(c, st, c->vpk2[0], w, rows, &nsplit, &pstride));
+        TRY(launch_panel_gram(c, st, c->vpk2[0], w, g.rows, &nsplit, &pstride));
         pre(c, st);
         k_wreduce4<<<(WP * WP * 4) / 256, 256, 0, st>>>(w.wpart, pstride, nsplit, (int64_t)WP * WP, w.wsum + (size_t)p * WP * WP);
         TRY(post(c, st, "k_wreduce4"));
@@ -1146,15 +1167,17 @@ static int apply_qt_local_vec(dhqr_context* c, cudaStream_t st, int64_t m, int64
 }
 static bool qt_vec_ok(const dhqr_context* c, int64_t m, int nrhs) { return c->qt_vec && nrhs == 1 && m <= (int64_t)QT_MAXG * QT_MAXROWS; }
 
+static constexpr size_t BS_BLOCK_WORDS = 32 * 2;   // k_backsolve_wave cells of one 32-row block: 32 cells of 2 words
+
 static int backsolve_local(dhqr_context* c, cudaStream_t st, int64_t col0, int64_t nl, const double* A, int64_t lda,
                            const double* alpha, double* y, int64_t ldy, int nrhs, double* x, int64_t ldx) {
     if (nl <= 0) return 0;
     // one launch per right-hand side: a wavefront over 32-row strips (k_backsolve_wave); needs every CTA resident at once
     const int64_t nbk = (nl + 31) / 32, nlow = (col0 + 31) / 32;
-    if (nbk + nlow <= c->bs_wave_max_ctas && nbk <= (int64_t)c->bs_cells_blocks) {
+    if (nbk + nlow <= c->bs_wave_max_ctas && nbk <= (int64_t)(c->bs_cells.size() / BS_BLOCK_WORDS)) {
         for (int rhs = 0; rhs < nrhs; ++rhs) {
             if (c->bs_epoch > 0xFFFFFFF0u) {
-                CU(cudaMemsetAsync(c->bs_cells, 0, (size_t)c->bs_cells_blocks * 32 * 16, st));
+                CU(cudaMemsetAsync(c->bs_cells, 0, sizeof(unsigned long long) * c->bs_cells.size(), st));
                 c->bs_epoch = 0;
             }
             k_backsolve_wave<<<(unsigned)(nbk + nlow), BW_THREADS, 0, st>>>(A, lda, alpha, y + (int64_t)rhs * ldy, x + (int64_t)rhs * ldx, col0, nl,
@@ -1174,6 +1197,53 @@ static int backsolve_local(dhqr_context* c, cudaStream_t st, int64_t col0, int64
     return 0;
 }
 
+// The options of dhqr_set_option / dhqr_get_option (documented in include/dhqr.h).  A flag stores any nonzero value as 1;
+// a bounded option refuses, with range_err, a value outside [lo, hi] or not a multiple of mult; wide_kappa is a double
+// read back truncated; a read-only option has a getter instead of a member.
+struct OptionDef {
+    const char* key;
+    enum Kind { FLAG, INT, REAL, READ_ONLY } kind;
+    int dhqr_context::*ival;                   // FLAG, INT
+    double dhqr_context::*dval;                // REAL
+    int64_t lo, hi, mult;                      // INT, REAL
+    const char* range_err;                     // INT, REAL
+    int (*get)(dhqr_context*, int64_t*);       // READ_ONLY
+};
+static int get_fast_stat(dhqr_context* c, int which, int64_t* value) {
+    int st2[2] = {0, 0};
+    if (c->fast_stats) CU(cudaMemcpy(st2, c->fast_stats, sizeof(st2), cudaMemcpyDeviceToHost));
+    *value = st2[which];
+    return 0;
+}
+static const OptionDef OPTIONS[] = {
+    {"nb", OptionDef::INT, &dhqr_context::nb, nullptr, 32, 128, 32, "nb must be a multiple of 32 in [32,128]"},
+    {"sync", OptionDef::FLAG, &dhqr_context::sync},
+    {"profile", OptionDef::FLAG, &dhqr_context::profile},
+    {"lookahead", OptionDef::FLAG, &dhqr_context::lookahead},
+    {"host_trace", OptionDef::FLAG, &dhqr_context::host_trace},
+    {"host_chunk", OptionDef::INT, &dhqr_context::host_chunk, nullptr, 0, INT64_MAX, 128, "host_chunk must be a non-negative multiple of 128"},
+    {"host_first", OptionDef::INT, &dhqr_context::host_first, nullptr, 0, INT64_MAX, 1, "host_first < 0"},
+    {"host_h2d_gbs", OptionDef::INT, &dhqr_context::host_h2d_gbs, nullptr, 1, INT64_MAX, 1, "host_h2d_gbs < 1"},
+    {"host_chain_us", OptionDef::INT, &dhqr_context::host_chain_us, nullptr, 1, INT64_MAX, 1, "host_chain_us < 1"},
+    {"host_tflops", OptionDef::INT, &dhqr_context::host_tflops, nullptr, 1, INT64_MAX, 1, "host_tflops < 1"},
+    {"qt_vec", OptionDef::FLAG, &dhqr_context::qt_vec},
+    {"panel_fast", OptionDef::FLAG, &dhqr_context::panel_fast},
+    {"wide_panel", OptionDef::FLAG, &dhqr_context::wide_panel},
+    {"wide_kappa", OptionDef::REAL, nullptr, &dhqr_context::wide_kappa, 1, INT64_MAX, 1, "wide_kappa < 1"},
+    {"wide_panels", OptionDef::READ_ONLY, nullptr, nullptr, 0, 0, 0, nullptr, [](dhqr_context* c, int64_t* v) { *v = c->wide_panels; return 0; }},
+    {"wide_redone", OptionDef::READ_ONLY, nullptr, nullptr, 0, 0, 0, nullptr, [](dhqr_context* c, int64_t* v) { *v = c->wide_redone; return 0; }},
+    {"panels_fast", OptionDef::READ_ONLY, nullptr, nullptr, 0, 0, 0, nullptr, [](dhqr_context* c, int64_t* v) { return get_fast_stat(c, 0, v); }},
+    {"panels_fallback", OptionDef::READ_ONLY, nullptr, nullptr, 0, 0, 0, nullptr, [](dhqr_context* c, int64_t* v) { return get_fast_stat(c, 1, v); }},
+    {"sms", OptionDef::READ_ONLY, nullptr, nullptr, 0, 0, 0, nullptr, [](dhqr_context* c, int64_t* v) { *v = c->sms; return 0; }},
+    {"rank", OptionDef::READ_ONLY, nullptr, nullptr, 0, 0, 0, nullptr, [](dhqr_context* c, int64_t* v) { *v = c->rank; return 0; }},
+    {"nranks", OptionDef::READ_ONLY, nullptr, nullptr, 0, 0, 0, nullptr, [](dhqr_context* c, int64_t* v) { *v = c->nranks; return 0; }},
+};
+static const OptionDef* find_option(const char* key) {
+    for (const OptionDef& o : OPTIONS)
+        if (!strcmp(o.key, key)) return &o;
+    return nullptr;
+}
+
 // ------------------------------------------------------------------------------------------------
 // C-ABI
 // ------------------------------------------------------------------------------------------------
@@ -1191,24 +1261,24 @@ static int create_common(dhqr_handle* h, int device) {
     cudaDeviceProp prop;
     CU(cudaGetDeviceProperties(&prop, device));
     if (prop.major < 10) return set_err(5001, "libdhqr is built for sm_100a only; device %d is sm_%d%d", device, prop.major, prop.minor);
-    dhqr_context* c = new dhqr_context();
+    std::unique_ptr<dhqr_context> c(new dhqr_context());   // a failure below releases what was made so far
     c->device = device;
     c->sms = prop.multiProcessorCount;
-    CU(cudaMalloc((void**)&c->d_i64, sizeof(int64_t) * 2 * 1025));
-    CU(cudaStreamCreateWithFlags(&c->copy_stream, cudaStreamNonBlocking));
-    CU(cudaStreamCreateWithFlags(&c->d2h_stream, cudaStreamNonBlocking));
-    CU(cudaStreamCreateWithFlags(&c->h2d_stream, cudaStreamNonBlocking));
-    for (int i = 0; i < CU_STREAMS; ++i) CU(cudaStreamCreateWithFlags(&c->cu_stream[i], cudaStreamNonBlocking));
+    TRY(c->d_i64.grow(2 * 1025));
+    CU(c->copy_stream.create());
+    CU(c->d2h_stream.create());
+    CU(c->h2d_stream.create());
+    for (int i = 0; i < CU_STREAMS; ++i) CU(c->cu_stream[i].create());
     {
         int lo = 0, hi = 0;
         CU(cudaDeviceGetStreamPriorityRange(&lo, &hi));
-        CU(cudaStreamCreateWithPriority(&c->hp_stream, cudaStreamNonBlocking, hi));
-        CU(cudaStreamCreateWithPriority(&c->comm_stream, cudaStreamNonBlocking, hi));
-        CU(cudaStreamCreateWithPriority(&c->hp2_stream, cudaStreamNonBlocking, hi));
-        CU(cudaStreamCreateWithPriority(&c->aux_stream, cudaStreamNonBlocking, hi));
-        for (int i = 0; i < 4; ++i) CU(cudaEventCreateWithFlags(&c->ev_aux[i], cudaEventDisableTiming));
+        CU(c->hp_stream.create(hi));
+        CU(c->comm_stream.create(hi));
+        CU(c->hp2_stream.create(hi));
+        CU(c->aux_stream.create(hi));
+        for (int i = 0; i < 4; ++i) CU(c->ev_aux[i].create(cudaEventDisableTiming));
     }
-    *h = c;
+    *h = c.release();
     return 0;
 }
 
@@ -1245,71 +1315,22 @@ int dhqr_destroy(dhqr_handle c) {
     cudaSetDevice(c->device);
     cudaDeviceSynchronize();
     if (c->comm) g_nccl.CommDestroy(c->comm);
-    cudaFree(c->linv_all);
-    for (int b = 0; b < 3 + CU_STREAMS; ++b) {
-        cudaFree(c->vpk2[b]);
-        cudaFree(c->ws[b].wpart); cudaFree(c->ws[b].wsum); cudaFree(c->ws[b].ypk); cudaFree(c->ws[b].linv);
-    }
-    cudaFree(c->uw_flags);
-    cudaFree(c->qt_T); cudaFree(c->qt_part); cudaFree(c->qt_ticket);
-    cudaFree(c->wctl); cudaFree(c->wbuf); cudaFree(c->bs_cells);
-    cudaFree(c->cells); cudaFree(c->cells2); cudaFree(c->fast_stats);
-    if (c->hp_stream) cudaStreamDestroy(c->hp_stream);
-    if (c->comm_stream) cudaStreamDestroy(c->comm_stream);
-    if (c->hp2_stream) cudaStreamDestroy(c->hp2_stream);
-    if (c->aux_stream) cudaStreamDestroy(c->aux_stream);
-    for (int i = 0; i < 4; ++i)
-        if (c->ev_aux[i]) cudaEventDestroy(c->ev_aux[i]);
-    cudaFree(c->v1); cudaFree(c->xbuf); cudaFree(c->hostA); cudaFree(c->hostB); cudaFree(c->d_i64);
-    if (c->copy_stream) cudaStreamDestroy(c->copy_stream);
-    if (c->d2h_stream) cudaStreamDestroy(c->d2h_stream);
-    if (c->h2d_stream) cudaStreamDestroy(c->h2d_stream);
-    for (int i = 0; i < CU_STREAMS; ++i) if (c->cu_stream[i]) cudaStreamDestroy(c->cu_stream[i]);
-    delete c;
+    delete c;   // the owners release every buffer, stream and event
     return 0;
 }
 
 int dhqr_set_option(dhqr_handle c, const char* key, int64_t value) {
     if (!c) return set_err(-1, "null handle");
     if (!key) return set_err(-2, "null key");
-    if (!strcmp(key, "nb")) {
-        if (value < 32 || value > 128 || value % 32) return set_err(-3, "nb must be a multiple of 32 in [32,128]");
-        c->nb = (int)value;
-    } else if (!strcmp(key, "sync")) {
-        c->sync = value ? 1 : 0;
-    } else if (!strcmp(key, "profile")) {
-        c->profile = value ? 1 : 0;
-    } else if (!strcmp(key, "lookahead")) {
-        c->lookahead = value ? 1 : 0;
-    } else if (!strcmp(key, "host_trace")) {
-        c->host_trace = value ? 1 : 0;
-    } else if (!strcmp(key, "host_chunk")) {
-        if (value < 0 || value % 128) return set_err(-3, "host_chunk must be a non-negative multiple of 128");
-        c->host_chunk = (int)value;
-    } else if (!strcmp(key, "host_first")) {
-        if (value < 0) return set_err(-3, "host_first < 0");
-        c->host_first = (int)value;
-    } else if (!strcmp(key, "host_h2d_gbs")) {
-        if (value < 1) return set_err(-3, "host_h2d_gbs < 1");
-        c->host_h2d_gbs = (int)value;
-    } else if (!strcmp(key, "host_chain_us")) {
-        if (value < 1) return set_err(-3, "host_chain_us < 1");
-        c->host_chain_us = (int)value;
-    } else if (!strcmp(key, "host_tflops")) {
-        if (value < 1) return set_err(-3, "host_tflops < 1");
-        c->host_tflops = (int)value;
-    } else if (!strcmp(key, "qt_vec")) {
-        c->qt_vec = value ? 1 : 0;
-    } else if (!strcmp(key, "panel_fast")) {
-        c->panel_fast = value ? 1 : 0;
-    } else if (!strcmp(key, "wide_panel")) {
-        c->wide_panel = value ? 1 : 0;
-    } else if (!strcmp(key, "wide_kappa")) {
-        if (value < 1) return set_err(-3, "wide_kappa < 1");
-        c->wide_kappa = (double)value;
-    } else {
-        return set_err(-2, "unknown option '%s'", key);
+    const OptionDef* o = find_option(key);
+    if (!o || o->kind == OptionDef::READ_ONLY) return set_err(-2, "unknown option '%s'", key);
+    if (o->kind == OptionDef::FLAG) {
+        c->*o->ival = value ? 1 : 0;
+        return 0;
     }
+    if (value < o->lo || value > o->hi || value % o->mult) return set_err(-3, "%s", o->range_err);
+    if (o->kind == OptionDef::REAL) c->*o->dval = (double)value;
+    else c->*o->ival = (int)value;
     return 0;
 }
 
@@ -1317,31 +1338,10 @@ int dhqr_get_option(dhqr_handle c, const char* key, int64_t* value) {
     if (!c) return set_err(-1, "null handle");
     if (!key) return set_err(-2, "null key");
     if (!value) return set_err(-3, "null value");
-    if (!strcmp(key, "nb")) *value = c->nb;
-    else if (!strcmp(key, "lookahead")) *value = c->lookahead;
-    else if (!strcmp(key, "wide_panel")) *value = c->wide_panel;
-    else if (!strcmp(key, "wide_kappa")) *value = (int64_t)c->wide_kappa;
-    else if (!strcmp(key, "panel_fast")) *value = c->panel_fast;
-    else if (!strcmp(key, "qt_vec")) *value = c->qt_vec;
-    else if (!strcmp(key, "host_chunk")) *value = c->host_chunk;
-    else if (!strcmp(key, "host_first")) *value = c->host_first;
-    else if (!strcmp(key, "host_h2d_gbs")) *value = c->host_h2d_gbs;
-    else if (!strcmp(key, "host_tflops")) *value = c->host_tflops;
-    else if (!strcmp(key, "host_chain_us")) *value = c->host_chain_us;
-    else if (!strcmp(key, "host_trace")) *value = c->host_trace;
-    else if (!strcmp(key, "sync")) *value = c->sync;
-    else if (!strcmp(key, "profile")) *value = c->profile;
-    else if (!strcmp(key, "wide_panels")) *value = c->wide_panels;
-    else if (!strcmp(key, "wide_redone")) *value = c->wide_redone;
-    else if (!strcmp(key, "panels_fast") || !strcmp(key, "panels_fallback")) {
-        int st2[2] = {0, 0};
-        if (c->fast_stats) CU(cudaMemcpy(st2, c->fast_stats, sizeof(st2), cudaMemcpyDeviceToHost));
-        *value = st2[!strcmp(key, "panels_fallback") ? 1 : 0];
-    }
-    else if (!strcmp(key, "sms")) *value = c->sms;
-    else if (!strcmp(key, "rank")) *value = c->rank;
-    else if (!strcmp(key, "nranks")) *value = c->nranks;
-    else return set_err(-2, "unknown option '%s'", key);
+    const OptionDef* o = find_option(key);
+    if (!o) return set_err(-2, "unknown option '%s'", key);
+    if (o->kind == OptionDef::READ_ONLY) return o->get(c, value);
+    *value = o->kind == OptionDef::REAL ? (int64_t)(c->*o->dval) : c->*o->ival;
     return 0;
 }
 
@@ -1359,8 +1359,6 @@ static int prof_drain(dhqr_context* c) {
         CU(cudaEventElapsedTime(&ms, r.e0, r.e1));
         c->prof_slots[r.slot].ms += ms;
         c->prof_slots[r.slot].count += 1;
-        cudaEventDestroy(r.e0);
-        cudaEventDestroy(r.e1);
     }
     c->prof_pending.clear();
     return 0;
@@ -1398,12 +1396,12 @@ int dhqr_qr_f64(dhqr_handle c, int64_t m, int64_t n_global, int64_t col0, int64_
     return qr_blocked(c, st, m, n_global, col0, n_local, dA, lda, d_alpha, nb);
 }
 
-int dhqr_apply_qt_f64(dhqr_handle c, int64_t m, int64_t n_global, int64_t col0, int64_t n_local, const double* dA,
-                      int64_t lda, double* d_b, int64_t ldb, int nrhs, void* stream) {
+// b <- Q'b (notrans = 0; C3, S:227-229: the owners act on b one after the other, b travels rank -> rank + 1) or
+// b <- Qb = H_1 ... H_n b (notrans = 1: the owners act in reverse rank order, b travels rank -> rank - 1)
+static int apply_q_sweep(dhqr_context* c, int64_t m, int64_t n_global, int64_t col0, int64_t n_local, const double* dA, int64_t lda,
+                         double* d_b, int64_t ldb, int nrhs, void* stream, int notrans) {
     TRY(check_common(c, m, n_global, col0, n_local, dA, lda));
-    if (nrhs < 0) return set_err(-10, "nrhs < 0");
-    if (nrhs > 0 && !d_b) return set_err(-8, "null b");
-    if (ldb < std::max<int64_t>(1, m)) return set_err(-9, "ldb < max(1,m)");
+    TRY(check_rhs(m, nrhs, d_b, ldb, 8, 9, 10));
     if (n_global == 0 || nrhs == 0) return 0;
     CU(cudaSetDevice(c->device));
     cudaStream_t st = (cudaStream_t)stream;
@@ -1411,69 +1409,47 @@ int dhqr_apply_qt_f64(dhqr_handle c, int64_t m, int64_t n_global, int64_t col0, 
     TRY(gather_partition(c, st, col0, n_local, col0s, nls));
     TRY(check_partition(col0s, nls, n_global));
     TRY(ensure_workspace(c, m, std::max<int64_t>(n_local, nrhs)));
-    // C3 (S:227-229): owners act on b one after the other; b travels rank -> rank
+    const int from = notrans ? c->rank + 1 : c->rank - 1, to = notrans ? c->rank - 1 : c->rank + 1;
+    const int last = notrans ? 0 : c->nranks - 1;   // the rank that finishes b
     const size_t cnt = (size_t)ldb * (nrhs - 1) + m;
     const bool vec = qt_vec_ok(c, m, nrhs);
     if (vec) TRY(qt_prepare(c, st, m, col0, n_local, dA, lda));
-    if (c->nranks > 1 && c->rank > 0) NC(g_nccl.Recv(d_b, cnt, ncclFloat64, c->rank - 1, c->comm, st));
-    if (vec) TRY(apply_qt_local_vec(c, st, m, col0, n_local, dA, lda, d_b, 0));
-    else TRY(apply_qt_local(c, st, m, col0, n_local, dA, lda, d_b, ldb, nrhs));
+    if (c->nranks > 1 && from >= 0 && from < c->nranks) NC(g_nccl.Recv(d_b, cnt, ncclFloat64, from, c->comm, st));
+    if (vec) TRY(apply_qt_local_vec(c, st, m, col0, n_local, dA, lda, d_b, notrans));
+    else TRY(apply_qt_local(c, st, m, col0, n_local, dA, lda, d_b, ldb, nrhs, notrans));
     if (c->nranks > 1) {
-        if (c->rank + 1 < c->nranks) NC(g_nccl.Send(d_b, cnt, ncclFloat64, c->rank + 1, c->comm, st));
-        NC(g_nccl.Broadcast(d_b, d_b, cnt, ncclFloat64, c->nranks - 1, c->comm, st));
+        if (to >= 0 && to < c->nranks) NC(g_nccl.Send(d_b, cnt, ncclFloat64, to, c->comm, st));
+        NC(g_nccl.Broadcast(d_b, d_b, cnt, ncclFloat64, last, c->comm, st));
     }
     return 0;
 }
 
+int dhqr_apply_qt_f64(dhqr_handle c, int64_t m, int64_t n_global, int64_t col0, int64_t n_local, const double* dA,
+                      int64_t lda, double* d_b, int64_t ldb, int nrhs, void* stream) {
+    return apply_q_sweep(c, m, n_global, col0, n_local, dA, lda, d_b, ldb, nrhs, stream, 0);
+}
+
 int dhqr_apply_q_f64(dhqr_handle c, int64_t m, int64_t n_global, int64_t col0, int64_t n_local, const double* dA,
                      int64_t lda, double* d_b, int64_t ldb, int nrhs, void* stream) {
-    TRY(check_common(c, m, n_global, col0, n_local, dA, lda));
-    if (nrhs < 0) return set_err(-10, "nrhs < 0");
-    if (nrhs > 0 && !d_b) return set_err(-8, "null b");
-    if (ldb < std::max<int64_t>(1, m)) return set_err(-9, "ldb < max(1,m)");
-    if (n_global == 0 || nrhs == 0) return 0;
-    CU(cudaSetDevice(c->device));
-    cudaStream_t st = (cudaStream_t)stream;
-    std::vector<int64_t> col0s, nls;
-    TRY(gather_partition(c, st, col0, n_local, col0s, nls));
-    TRY(check_partition(col0s, nls, n_global));
-    TRY(ensure_workspace(c, m, std::max<int64_t>(n_local, nrhs)));
-    // b <- H_1 ... H_n b: the owners act in reverse rank order, b travels rank -> rank - 1
-    const size_t cnt = (size_t)ldb * (nrhs - 1) + m;
-    const bool vec = qt_vec_ok(c, m, nrhs);
-    if (vec) TRY(qt_prepare(c, st, m, col0, n_local, dA, lda));
-    if (c->nranks > 1 && c->rank + 1 < c->nranks) NC(g_nccl.Recv(d_b, cnt, ncclFloat64, c->rank + 1, c->comm, st));
-    if (vec) TRY(apply_qt_local_vec(c, st, m, col0, n_local, dA, lda, d_b, 1));
-    else TRY(apply_qt_local(c, st, m, col0, n_local, dA, lda, d_b, ldb, nrhs, 1));
-    if (c->nranks > 1) {
-        if (c->rank > 0) NC(g_nccl.Send(d_b, cnt, ncclFloat64, c->rank - 1, c->comm, st));
-        NC(g_nccl.Broadcast(d_b, d_b, cnt, ncclFloat64, 0, c->comm, st));
-    }
-    return 0;
+    return apply_q_sweep(c, m, n_global, col0, n_local, dA, lda, d_b, ldb, nrhs, stream, 1);
 }
 
 int dhqr_backsolve_f64(dhqr_handle c, int64_t m, int64_t n_global, int64_t col0, int64_t n_local, const double* dA,
                        int64_t lda, const double* d_alpha, double* d_b, int64_t ldb, int nrhs, void* stream) {
     TRY(check_common(c, m, n_global, col0, n_local, dA, lda));
     if (n_global > 0 && !d_alpha) return set_err(-8, "null alpha");
-    if (nrhs < 0) return set_err(-11, "nrhs < 0");
-    if (nrhs > 0 && !d_b) return set_err(-9, "null b");
-    if (ldb < std::max<int64_t>(1, m)) return set_err(-10, "ldb < max(1,m)");
+    TRY(check_rhs(m, nrhs, d_b, ldb, 9, 10, 11));
     if (n_global == 0 || nrhs == 0) return 0;
     CU(cudaSetDevice(c->device));
     cudaStream_t st = (cudaStream_t)stream;
     std::vector<int64_t> col0s, nls;
     TRY(gather_partition(c, st, col0, n_local, col0s, nls));
     TRY(check_partition(col0s, nls, n_global));
-    TRY(ensure(&c->xbuf, &c->xbuf_elems, (size_t)n_global * nrhs));
-    if (c->bs_cells_blocks < (size_t)(n_local + 31) / 32 + 1) {
-        if (c->bs_cells) CU(cudaFree(c->bs_cells));
-        c->bs_cells = nullptr;
-        c->bs_cells_blocks = (size_t)(n_local + 31) / 32 + 64;
-        CU(cudaMalloc((void**)&c->bs_cells, c->bs_cells_blocks * 32 * 16));
-        CU(cudaMemset(c->bs_cells, 0, c->bs_cells_blocks * 32 * 16));
-        c->bs_epoch = 0;
-    }
+    TRY(c->xbuf.grow((size_t)n_global * nrhs));
+    const size_t blocks = (size_t)(n_local + 31) / 32;
+    bool fresh = false;   // new cells (64 blocks spare): the tags start over
+    if (c->bs_cells.size() < (blocks + 1) * BS_BLOCK_WORDS) TRY(c->bs_cells.grow((blocks + 64) * BS_BLOCK_WORDS, &fresh));
+    if (fresh) c->bs_epoch = 0;
     if (!c->bs_wave_max_ctas) {
         int per_sm = 0;
         CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_backsolve_wave, BW_THREADS, 0));
@@ -1557,9 +1533,7 @@ int dhqr_qr_c64(dhqr_handle c, int64_t m, int64_t n_global, int64_t col0, int64_
 int dhqr_apply_qt_c64(dhqr_handle c, int64_t m, int64_t n_global, int64_t col0, int64_t n_local, const void* dA, int64_t lda,
                       void* d_b, int64_t ldb, int nrhs, void* stream) {
     TRY(check_complex(c, m, n_global, col0, n_local, dA, lda));
-    if (nrhs < 0) return set_err(-10, "nrhs < 0");
-    if (nrhs > 0 && !d_b) return set_err(-8, "null b");
-    if (ldb < std::max<int64_t>(1, m)) return set_err(-9, "ldb < max(1,m)");
+    TRY(check_rhs(m, nrhs, d_b, ldb, 8, 9, 10));
     if (n_global == 0 || nrhs == 0) return 0;
     CU(cudaSetDevice(c->device));
     cudaStream_t st = (cudaStream_t)stream;
@@ -1579,16 +1553,14 @@ int dhqr_backsolve_c64(dhqr_handle c, int64_t m, int64_t n_global, int64_t col0,
                        const void* d_alpha, void* d_b, int64_t ldb, int nrhs, void* stream) {
     TRY(check_complex(c, m, n_global, col0, n_local, dA, lda));
     if (n_global > 0 && !d_alpha) return set_err(-8, "null alpha");
-    if (nrhs < 0) return set_err(-11, "nrhs < 0");
-    if (nrhs > 0 && !d_b) return set_err(-9, "null b");
-    if (ldb < std::max<int64_t>(1, m)) return set_err(-10, "ldb < max(1,m)");
+    TRY(check_rhs(m, nrhs, d_b, ldb, 9, 10, 11));
     if (n_global == 0 || nrhs == 0) return 0;
     CU(cudaSetDevice(c->device));
     cudaStream_t st = (cudaStream_t)stream;
     const int64_t n = n_global;
-    TRY(ensure(&c->xbuf, &c->xbuf_elems, (size_t)2 * n * nrhs));
+    TRY(c->xbuf.grow((size_t)2 * n * nrhs));
     const double2* A = (const double2*)dA;
-    double2* x = (double2*)c->xbuf;
+    double2* x = (double2*)(double*)c->xbuf;
     for (int64_t o = ((n - 1) / BS_BLK) * BS_BLK; o >= 0; o -= BS_BLK) {     // S:260: i = n:-1:1, by blocks
         const int bs = (int)std::min<int64_t>(BS_BLK, n - o);
         const int grid = (int)std::max<int64_t>(1, std::min<int64_t>((o + 255) / 256, 2 * c->sms));
@@ -1694,14 +1666,13 @@ int dhqr_qr_host_f64(dhqr_handle c, int64_t m, int64_t n, double* hA, int64_t ld
     if (blocked) plan_upload(&um, m, n, nbe, B, join);
     else { B = {0, n}; join = {0}; }
     const int nch = (int)B.size() - 1;
-    TRY(ensure(&c->hostA, &c->hostA_elems, (size_t)ldd * n + (size_t)n));
+    TRY(c->hostA.grow((size_t)ldd * n + (size_t)n));
     // everything sized once, before the pipeline starts: growing a buffer later would synchronise the device
     TRY(ensure_workspace(c, m, n, blocked ? (n + nbe - 1) / nbe + 1 : 0, nch > 1));
     double* dA = c->hostA;
     double* dal = c->hostA + (size_t)ldd * n;
     cudaStream_t st = c->copy_stream;
-    int rc = 0;
-    std::vector<cudaEvent_t> evUp;
+    std::vector<Event> evUp;
     struct timespec ts0;
     clock_gettime(CLOCK_MONOTONIC, &ts0);
     auto stamp = [&](const char* what, bool sync_all) {
@@ -1717,46 +1688,40 @@ int dhqr_qr_host_f64(dhqr_handle c, int64_t m, int64_t n, double* hA, int64_t ld
         fprintf(stderr, "\n");
     }
     c->up_chunks.clear();
-    do {
-        if (cudaMemcpy2DAsync(dA, (size_t)ldd * 8, hA, (size_t)lda * 8, (size_t)m * 8, (size_t)B[1], cudaMemcpyHostToDevice, st) != cudaSuccess) { rc = set_err(1001, "H2D failed"); break; }
+    const int rc = [&]() -> int {
+        CU(cudaMemcpy2DAsync(dA, (size_t)ldd * 8, hA, (size_t)lda * 8, (size_t)m * 8, (size_t)B[1], cudaMemcpyHostToDevice, st));
         if (nch > 1) {
             // the later chunks go up one after the other BEHIND the first (concurrent uploads would share the link and delay the
             // start of the factorisation), on their own stream
-            cudaEvent_t e0;
-            if (cudaEventCreateWithFlags(&e0, cudaEventDisableTiming) != cudaSuccess) { rc = set_err(1001, "event create failed"); break; }
-            evUp.push_back(e0);
-            cudaEventRecord(e0, st);
-            cudaStreamWaitEvent(c->h2d_stream, e0, 0);
-            for (int j = 1; j < nch && !rc; ++j) {
-                cudaEvent_t e;
-                if (cudaEventCreateWithFlags(&e, c->host_trace ? cudaEventDefault : cudaEventDisableTiming) != cudaSuccess) { rc = set_err(1001, "event create failed"); break; }
-                evUp.push_back(e);
-                if (cudaMemcpy2DAsync(dA + B[j] * ldd, (size_t)ldd * 8, hA + B[j] * lda, (size_t)lda * 8, (size_t)m * 8, (size_t)(B[j + 1] - B[j]),
-                                      cudaMemcpyHostToDevice, c->h2d_stream) != cudaSuccess) { rc = set_err(1001, "H2D failed"); break; }
-                cudaEventRecord(e, c->h2d_stream);
+            Event& e0 = evUp.emplace_back();
+            CU(e0.create(cudaEventDisableTiming));
+            CU(cudaEventRecord(e0, st));
+            CU(cudaStreamWaitEvent(c->h2d_stream, e0, 0));
+            for (int j = 1; j < nch; ++j) {
+                Event& e = evUp.emplace_back();
+                CU(e.create(c->host_trace ? cudaEventDefault : cudaEventDisableTiming));
+                CU(cudaMemcpy2DAsync(dA + B[j] * ldd, (size_t)ldd * 8, hA + B[j] * lda, (size_t)lda * 8, (size_t)m * 8, (size_t)(B[j + 1] - B[j]),
+                                     cudaMemcpyHostToDevice, c->h2d_stream));
+                CU(cudaEventRecord(e, c->h2d_stream));
                 c->up_chunks.push_back({B[j], B[j + 1], e, join[j]});
             }
-            if (rc) break;
         }
         stamp("first chunk uploaded", true);
         if (blocked) { c->mirror_host = hA; c->mirror_lda = lda; }   // finished panels stream back while later panels are factored
-        rc = dhqr_qr_f64(c, m, n, 0, n, dA, ldd, dal, nb, st);
-        c->mirror_host = nullptr;
-        if (rc) break;
+        TRY(dhqr_qr_f64(c, m, n, 0, n, dA, ldd, dal, nb, st));
         stamp("factored", true);
-        if (!blocked)
-            if (cudaMemcpy2DAsync(hA, (size_t)lda * 8, dA, (size_t)ldd * 8, (size_t)m * 8, (size_t)n, cudaMemcpyDeviceToHost, st) != cudaSuccess) { rc = set_err(1001, "D2H failed"); break; }
-        if (cudaMemcpyAsync(h_alpha, dal, (size_t)n * 8, cudaMemcpyDeviceToHost, st) != cudaSuccess) { rc = set_err(1001, "D2H failed"); break; }
-    } while (0);
+        if (!blocked) CU(cudaMemcpy2DAsync(hA, (size_t)lda * 8, dA, (size_t)ldd * 8, (size_t)m * 8, (size_t)n, cudaMemcpyDeviceToHost, st));
+        CU(cudaMemcpyAsync(h_alpha, dal, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
+        return 0;
+    }();
+    // on every exit of the pipeline: nothing of it may still run (or still write to hA) when the call returns
     c->mirror_host = nullptr;
     c->up_chunks.clear();
     cudaError_t e0 = cudaStreamSynchronize(c->h2d_stream), e1 = cudaStreamSynchronize(st), e2 = cudaStreamSynchronize(c->d2h_stream);
     cudaError_t e3 = cudaSuccess;
     for (int i = 0; i < CU_STREAMS; ++i) { const cudaError_t e4 = cudaStreamSynchronize(c->cu_stream[i]); if (e3 == cudaSuccess) e3 = e4; }
     stamp("everything back on the host", false);
-    for (cudaEvent_t ev : c->panel_events) cudaEventDestroy(ev);
     c->panel_events.clear();
-    for (cudaEvent_t ev : evUp) cudaEventDestroy(ev);
     if (rc) return rc;
     if (e0 != cudaSuccess) return set_err(1000 + (int)e0, "qr_host H2D: %s", cudaGetErrorString(e0));
     if (e1 != cudaSuccess) return set_err(1000 + (int)e1, "qr_host: %s", cudaGetErrorString(e1));
@@ -1775,8 +1740,8 @@ int dhqr_ldiv_host_f64(dhqr_handle c, int64_t m, int64_t n, const double* hA, in
     if (n == 0) return 0;
     CU(cudaSetDevice(c->device));
     const int64_t ldd = rup(m, 32);
-    TRY(ensure(&c->hostA, &c->hostA_elems, (size_t)ldd * n + (size_t)n));
-    TRY(ensure(&c->hostB, &c->hostB_elems, (size_t)ldd));
+    TRY(c->hostA.grow((size_t)ldd * n + (size_t)n));
+    TRY(c->hostB.grow((size_t)ldd));
     double* dA = c->hostA;
     double* dal = c->hostA + (size_t)ldd * n;
     cudaStream_t st = c->copy_stream;
@@ -1832,10 +1797,7 @@ int dhqr_k_block_reflector_f64(dhqr_handle c, int64_t rows, int nbp, const doubl
     cudaStream_t st = (cudaStream_t)stream;
     TRY(ensure_workspace(c, rows, ncols));
     const int nbk = nbp <= IB ? IB : NBMAX;
-    const int64_t vrows = rup(rows, 128);
-    dim3 grid((unsigned)std::min<int64_t>((vrows / 4 + 255) / 256, 4 * c->sms), nbk);
-    k_pack<<<grid, 256, 0, st>>>(dV, ldv, rows, nbp, 0, c->vpk2[0], 0, 0, vrows);
-    TRY(post(c, st, "k_pack"));
+    TRY(pack_panel(c, st, dV, ldv, rows, nbp, 0, c->vpk2[0], 0, panel_geom({0, 0, nbp}, rows).vrows, nbk));
     TRY(apply_block_reflector(c, st, c->vpk2[0], c->ws[0], 0, nbk, rows, row_lo, dC, ldc, ncols));
     if (d_linv_out) CU(cudaMemcpyAsync(d_linv_out, c->ws[0].linv, sizeof(double) * (size_t)nbk * nbk, cudaMemcpyDeviceToDevice, st));
     return 0;
@@ -1847,12 +1809,12 @@ int dhqr_debug_copy_f64(dhqr_handle c, const char* which, double* d_dst, int64_t
     if (!d_dst) return set_err(-3, "null destination");
     const double* src = nullptr;
     size_t have = 0;
-    if (!strcmp(which, "wpart")) { src = c->ws[0].wpart; have = c->ws[0].wpart_elems; }
-    else if (!strcmp(which, "wsum")) { src = c->ws[0].wsum; have = c->ws[0].wsum_elems; }
-    else if (!strcmp(which, "ypk")) { src = c->ws[0].ypk; have = c->ws[0].ypk_elems; }
+    if (!strcmp(which, "wpart")) { src = c->ws[0].wpart; have = c->ws[0].wpart.size(); }
+    else if (!strcmp(which, "wsum")) { src = c->ws[0].wsum; have = c->ws[0].wsum.size(); }
+    else if (!strcmp(which, "ypk")) { src = c->ws[0].ypk; have = c->ws[0].ypk.size(); }
     else if (!strcmp(which, "linv")) { src = c->ws[0].linv; have = (size_t)NBMAX * NBMAX; }
-    else if (!strcmp(which, "vpk")) { src = c->vpk2[0]; have = c->vpk_elems[0]; }
-    else if (!strcmp(which, "wide")) { src = c->wbuf; have = c->wbuf ? (size_t)5 * WP * WP + 3 * XL_ELEMS : 0; }
+    else if (!strcmp(which, "vpk")) { src = c->vpk2[0]; have = c->vpk2[0].size(); }
+    else if (!strcmp(which, "wide")) { src = c->wbuf; have = c->wbuf.size(); }
     else return set_err(-2, "unknown buffer '%s'", which);
     if (nelems < 0 || (size_t)nelems > have) return set_err(-4, "nelems out of range (have %zu)", have);
     CU(cudaMemcpyAsync(d_dst, src, sizeof(double) * (size_t)nelems, cudaMemcpyDeviceToDevice, (cudaStream_t)stream));

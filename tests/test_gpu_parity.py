@@ -300,6 +300,40 @@ def test_option_keys(D, key):
         assert e.value.code == -2
 
 
+# Values each bounded option refuses (include/dhqr.h gives the ranges); the other settable options are flags.
+OPTION_OUT_OF_RANGE = {"nb": [0, 16, 48, 160], "host_chunk": [-128, 100], "host_first": [-1], "host_h2d_gbs": [0, -1],
+                       "host_tflops": [0], "host_chain_us": [0], "wide_kappa": [0, -1000]}
+READ_ONLY_OPTIONS = ["sms", "rank", "nranks", "panels_fast", "panels_fallback", "wide_panels", "wide_redone"]
+
+
+@pytest.mark.parametrize("key", sorted(OPTION_DEFAULTS) + READ_ONLY_OPTIONS)
+def test_option_values(D, key):
+    # a bounded option refuses a value out of range with -3 and keeps the one it had; a flag stores any nonzero value as 1;
+    # a read-only key reads but refuses to be set (-2)
+    h = D.default_handle(0)
+    if key in READ_ONLY_OPTIONS:
+        v = h.get_option(key)
+        with pytest.raises(D._lib.DhqrError) as e:
+            h.set_option(key, v)
+        assert e.value.code == -2
+        assert h.get_option(key) == v
+        return
+    try:
+        h.set_option(key, OPTION_DEFAULTS[key])
+        if key in OPTION_OUT_OF_RANGE:
+            for bad in OPTION_OUT_OF_RANGE[key]:
+                with pytest.raises(D._lib.DhqrError) as e:
+                    h.set_option(key, bad)
+                assert e.value.code == -3, bad
+                assert h.get_option(key) == OPTION_DEFAULTS[key]
+        else:
+            for v, stored in ((5, 1), (-1, 1), (0, 0), (1, 1)):
+                h.set_option(key, v)
+                assert h.get_option(key) == stored, v
+    finally:
+        h.set_option(key, OPTION_DEFAULTS[key])
+
+
 def test_block_reflector_kernels(D, dev, oracle):
     # gemm_vta + tinv + ymake + gemm_cvy in isolation against torch fp64 on genuine Householder blocks
     h = D.default_handle(0)
